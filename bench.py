@@ -329,6 +329,25 @@ def run_reference(args, cfg):
 
 
 # ----------------------------------------------------------------------------------------------- B200 arm
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """--dump-outputs: what the timed path computed in its last step, one float64 DIR/<name>.npy per array (first axis = game),
+    so that two builds run with the same arguments can be compared output for output.  game_index.npy holds the game of every
+    row: all games, or, when the files would exceed DUMP_LIMIT_BYTES in all, a fixed sample (numpy PCG64 seed 0).  With
+    several ranks every rank writes its own shard under a _rank<r> suffix, within its share of the limit."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))
+    keep = min(n, (DUMP_LIMIT_BYTES // world - 4096) // row_bytes)          # 4096: room for the .npy headers
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    suffix = "" if world == 1 else "_rank%d" % rank
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "game_index%s.npy" % suffix), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, "%s%s.npy" % (name, suffix)), np.asarray(a)[idx].astype(np.float64))
+
+
 def run_b200(args, cfg):
     """Three passes over the SAME workload: the search is deterministic given the seeds (SURVEY N3), so every pass builds an
     identical engine from the same seeds, plays the same W warm-up moves and then the same K moves:
@@ -377,7 +396,7 @@ def run_b200(args, cfg):
     with Clocks(local_rank) as clk:
         eng.timer_start()
         for _ in range(args.steps):
-            eng.play_move(sims, auto_reset=True, want_stats=False)
+            actions, _ = eng.play_move(sims, auto_reset=True, want_stats=False)
         ms = eng.timer_stop()
     torch.cuda.synchronize()
     D.barrier()
@@ -385,6 +404,8 @@ def run_b200(args, cfg):
     longest_trace = c1.pop("max_trace_len", None)             # not cumulative: the longest trace of the last move
     c0.pop("max_trace_len", None)
     launches = sum(n for _, n in eng.phase_ms().values())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"actions": actions, "games": eng.get_games()}, rank, world)
     ms_max = D.max_over_ranks(ms, dev)
     delta = {k: c1[k] - c0[k] for k in c1}
     tot = D.sum_over_ranks(delta, dev)
@@ -652,7 +673,11 @@ def main():
                     help="b200_set_path_cache (memory traffic only, results identical): auto = the engine's default where it applies (LP mode, max_nodes <= 65536)")
     ap.add_argument("--ref-moves-per-step", type=int, default=2)
     ap.add_argument("--exchange-rows", type=int, default=131072, help="rows (212 B) of the fixed-size replay block each rank contributes to the per-move all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's actions and the games it left (get_games) as float64 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl b200 and --steps >= 1")
     if args.workload == "vanilla":
         G, sims, M, mode = args.games_per_gpu or 4096, args.sims or 300, args.max_nodes or 8192, "vanilla"
         name = "BASELINE configs[1]: Vanilla MCTS (random rollouts, no value net), %d games/GPU, %d sims/move" % (G, sims)

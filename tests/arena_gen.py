@@ -1,6 +1,8 @@
 """Seeded synthetic search arenas in the reference's array layout (agents/agent.py:58-88), per SURVEY §8(d):
 7-ary, depth 4-12, visit in [1,1000], value ~ U(0,50), variance ~ U(1,100), score non-decreasing along edges,
 10-30 % duplicated observations among siblings."""
+import zlib
+
 import numpy as np
 
 
@@ -84,6 +86,11 @@ def near_tie_arena(seed, M=64):
     return a
 
 
+def arena_crc(a):
+    """CRC-32 of an arena's arrays: ties a golden that stores only a seed to the exact arena the seed regenerates."""
+    return zlib.crc32(b"".join(np.ascontiguousarray(a[k]).tobytes() for k in ("child", "visit", "value", "variance", "score", "n2o")))
+
+
 def boards(n, seed):
     """tools/test.py:23-28 style inputs for the value network: random {0,1} cells, top rows cleared, four -1 cells."""
     rng = np.random.default_rng(seed)
@@ -110,6 +117,16 @@ def state_to_obskey(s):
     cells.sort()
     key[10] = np.uint32(sum(v << (8 * i) for i, v in enumerate(cells[:4])))
     return key
+
+
+def golden_bk_dist(z, p):
+    """node_dist after the backup of tests/golden/dist_golden.npz case prefix p: stored whole (bk_dist), or as the rows the backup
+    changed (bk_rows, bk_dist_rows) on top of the stored input node_dist."""
+    if p + "bk_dist" in z:
+        return z[p + "bk_dist"]
+    bk = z[p + "node_dist"].copy()
+    bk[z[p + "bk_rows"]] = z[p + "bk_dist_rows"]
+    return bk
 
 
 def make_dist_arena(seed, M=512, bins=50, max_depth=6, unvisited=0.0):

@@ -1,5 +1,6 @@
 """Generate tests/golden/*.npz by RUNNING THE REFERENCE ITSELF in the build container (it cannot travel to the GPU box):
   core_golden.npz     outputs of the reference's own agents/cppmodule/core.cpp (compiled unchanged -> oracle/_ref/core*.so)
+  core_live_golden.npz  the same core.cpp on 30 more arenas that tests/arena_gen.py regenerates from their seeds (only outputs stored)
   valuenet_golden.npz outputs of the reference's own model/model_vv.py Model_VV (torch CPU) with seeded weights
   dist_golden.npz     outputs of the reference's own numba cores agents/core_distributional.py (fastmath: pinned to 1e-5)
   agent_golden.npz    per-move statistics of the reference's own agents/ValueSimLP.py + agents/agent.py driving
@@ -23,7 +24,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path[:0] = [os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")]
 import oracle_py as O  # noqa: E402
-from arena_gen import make_arena, boards, state_to_obskey  # noqa: E402
+from arena_gen import arena_crc, make_arena, near_tie_arena, boards, state_to_obskey  # noqa: E402
 
 
 def gen_core(core):
@@ -67,6 +68,27 @@ def gen_core(core):
     out["n_cases"] = len(cases)
     np.savez_compressed(os.path.join(HERE, "core_golden.npz"), **out)
     print("core_golden: %d cases" % len(cases))
+
+
+def gen_core_live(core):
+    """core_live_golden.npz: select_trace_obs (low=1) and backup_trace_obs of the reference's own core.cpp on 30 arenas that
+    tests/arena_gen.py regenerates from their seeds (every observation visited, so check_low never draws rand()).  The arenas
+    are not stored, only their CRC-32; of the backed-up arrays only the entries the backup changed are stored (bk_idx)."""
+    out = {}
+    n = 30
+    for seed in range(n):
+        a = make_arena(1000 + seed, M=1024, max_depth=4 + seed % 7) if seed % 5 else near_tie_arena(seed)
+        p = "s%d_" % seed
+        tr = np.asarray(core.select_trace_obs(1, a["child"], a["visit"], a["value"], a["variance"], a["score"], a["n2o"], 1), np.int32)
+        b = {k: a[k].copy() for k in ("visit", "value", "variance")}
+        core.backup_trace_obs(tr, b["visit"], b["value"], b["variance"], a["n2o"], a["score"], 123.456, 7.89, 0.999)
+        idx = np.nonzero(np.logical_or.reduce([b[k] != a[k] for k in b]))[0].astype(np.int32)
+        out[p + "crc"], out[p + "trace"], out[p + "bk_idx"] = arena_crc(a), tr, idx
+        for k in b:
+            out[p + "bk_" + k] = b[k][idx]
+    out["n_cases"] = n
+    np.savez_compressed(os.path.join(HERE, "core_live_golden.npz"), **out)
+    print("core_live_golden: %d cases" % n)
 
 
 def gen_valuenet():
@@ -548,7 +570,12 @@ def gen_dist():
         ns, nd = a["node_stats"].copy(), a["node_dist"].copy()
         r = float(a["node_stats"][tr[-1], 2] + rng.uniform(0, 300))
         R.backup_trace_distributional(np.asarray(tr, np.int32), ns, nd, r, dist, 0.0, 5000.0)
-        out[p + "r"], out[p + "bk_stats"], out[p + "bk_dist"] = r, ns, nd
+        out[p + "r"], out[p + "bk_stats"] = r, ns
+        if i < n - 2:
+            out[p + "bk_dist"] = nd
+        else:   # keeps the file under 1 MB: only the rows the backup changed (the rest equal node_dist), see arena_gen.golden_bk_dist
+            rows = np.nonzero((nd != a["node_dist"]).any(axis=1))[0].astype(np.int32)
+            out[p + "bk_rows"], out[p + "bk_dist_rows"] = rows, nd[rows]
     out["n_cases"] = n
     np.savez_compressed(os.path.join(HERE, "dist_golden.npz"), **out)
     print("dist_golden: %d cases" % n)
@@ -587,8 +614,11 @@ if __name__ == "__main__":
         gen_agent_modes(pt)
     elif "--agent-cpp" in sys.argv:
         gen_agent_cpp(pt)
+    elif "--core-live" in sys.argv:
+        gen_core_live(core)
     else:
         gen_core(core)
+        gen_core_live(core)
         gen_valuenet()
         gen_agent(pt)
         gen_agent_explicit_gc(pt)

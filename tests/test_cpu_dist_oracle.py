@@ -4,6 +4,8 @@ import os
 
 import numpy as np
 
+from arena_gen import golden_bk_dist
+
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "dist_golden.npz")
 
 
@@ -19,4 +21,4 @@ def test_dist_oracle_matches_reference_numba(oracle):
         ns, nd = z[p + "node_stats"].copy(), z[p + "node_dist"].copy()
         oracle.backup_trace_distributional(z[p + "trace"], ns, nd, float(z[p + "r"]), z[p + "dist"], 0, 5000)
         assert np.allclose(ns, z[p + "bk_stats"], rtol=1e-5, atol=1e-5)
-        assert np.allclose(nd, z[p + "bk_dist"], rtol=1e-5, atol=1e-7)
+        assert np.allclose(nd, golden_bk_dist(z, p), rtol=1e-5, atol=1e-7)

@@ -1,12 +1,10 @@
-"""Pin the CPU oracle (oracle/*.c) to the reference: (a) against the committed golden vectors that were produced by
-running the reference itself (tests/golden/gen_golden.py), (b) when /root/reference is present, against the
-reference's own compiled core.cpp on fresh seeded arenas."""
+"""Pin the CPU oracle (oracle/*.c) to the reference: against the committed golden vectors that were produced by
+running the reference itself (tests/golden/gen_golden.py), on stored inputs and on seeded arenas regenerated here."""
 import os
 
 import numpy as np
-import pytest
 
-from arena_gen import make_arena, near_tie_arena, state_to_obskey
+from arena_gen import arena_crc, make_arena, near_tie_arena, state_to_obskey
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -205,18 +203,22 @@ def test_synthetic_eval_is_plain_integer_hash(oracle):
     assert 0 <= v < 64 and 0.5 <= var < 64.5 and v * 256 == int(v * 256) and (var - 0.5) * 16 == int((var - 0.5) * 16)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree absent (GPU box)")
 def test_live_against_reference_core(oracle):
-    oracle.build(ref=True)
-    _, core = oracle.mount_reference()
+    """select_trace_obs / backup_trace_obs on 30 seeded arenas vs what the reference's own compiled core.cpp returned on them
+    (tests/golden/gen_golden.py gen_core_live): the arenas are regenerated here, the golden holds their CRC-32 and the reference's
+    outputs.  The backed-up arrays must equal the reference's at the entries it changed and the input everywhere else."""
+    z = np.load(os.path.join(GOLD, "core_live_golden.npz"))
+    assert int(z["n_cases"]) == 30
     for seed in range(30):
+        p = "s%d_" % seed
         a = make_arena(1000 + seed, M=1024, max_depth=4 + seed % 7) if seed % 5 else near_tie_arena(seed)
-        tr = core.select_trace_obs(1, a["child"], a["visit"], a["value"], a["variance"], a["score"], a["n2o"], 1)
+        assert arena_crc(a) == int(z[p + "crc"]), "arena %d no longer matches the one the golden was recorded on" % seed
         mine = oracle.select_trace_obs(1, a["child"], a["visit"], a["value"], a["variance"], a["score"], a["n2o"], 1)
-        assert np.array_equal(np.asarray(tr), mine), seed
-        b1 = {k: a[k].copy() for k in ("visit", "value", "variance")}
+        assert np.array_equal(z[p + "trace"], mine), seed
         b2 = {k: a[k].copy() for k in ("visit", "value", "variance")}
-        core.backup_trace_obs(np.asarray(tr, np.int32), b1["visit"], b1["value"], b1["variance"], a["n2o"], a["score"], 123.456, 7.89, 0.999)
         oracle.backup_trace_obs(mine, b2["visit"], b2["value"], b2["variance"], a["n2o"], a["score"], 123.456, 7.89, 0.999)
-        for k in b1:
-            assert np.array_equal(b1[k], b2[k]), (seed, k)
+        idx = z[p + "bk_idx"]
+        for k in b2:
+            want = a[k].copy()
+            want[idx] = z[p + "bk_" + k]
+            assert np.array_equal(want, b2[k]), (seed, k)

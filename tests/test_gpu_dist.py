@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from arena_gen import make_dist_arena
+from arena_gen import golden_bk_dist, make_dist_arena
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden", "dist_golden.npz")
@@ -23,7 +23,7 @@ def test_dist_twins_match_reference_golden(gpu_lib):
         ns, nd = z[p + "node_stats"].copy(), z[p + "node_dist"].copy()
         CD.backup_trace_distributional(z[p + "trace"], ns, nd, float(z[p + "r"]), z[p + "dist"], 0, 5000)
         assert np.allclose(ns, z[p + "bk_stats"], rtol=1e-5, atol=1e-5)
-        assert np.allclose(nd, z[p + "bk_dist"], rtol=1e-5, atol=1e-7)
+        assert np.allclose(nd, golden_bk_dist(z, p), rtol=1e-5, atol=1e-7)
 
 
 def test_dist_twins_match_oracle_with_rng(gpu_lib, oracle):
