@@ -91,11 +91,6 @@ int b200_update_root(b200_engine *e, int auto_reset);
 int b200_remove_nodes(b200_engine *e, int min_free);
 int b200_set_gc_headroom(b200_engine *e, int min_free);
 
-/* --- scheduling only (no reference counterpart, no effect on any result): the up to max_games games whose last trace was longest walk the tree
- * on a second stream, so that a simulation step of the other games does not last as long as the deepest walk of all (ValueSim / ValueSimLP with
- * B200_EVAL_NET_TC; ignored otherwise).  0 (default) = one lane. */
-int b200_set_deep_lane(b200_engine *e, int max_games);
-
 /* --- memory traffic only (no reference counterpart, no effect on any result): the PATH CACHE.  Consecutive simulations of a game walk almost
  * the same root-to-leaf path (select_trace_obs, core.h:167-224, restarts at the root every time); with the cache on, a walk leaves next to its
  * trace the row fields and the children's statistics of every level, the backup (core.h:226-381) refreshes the copies it changes and drops

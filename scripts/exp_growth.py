@@ -10,9 +10,6 @@ moves = int(sys.argv[4]); ev = sys.argv[5] if len(sys.argv) > 5 else 'net'
 eng = BatchedEngine(G, max_nodes=M, mode='lp', eval_kind=ev, weights=init_weights(0), overflow_reset=True)
 eng.set_games(PT.new_games(G, (1, 0, 0), np.arange(123, 123 + G, dtype=np.uint32)))
 eng.set_gc_headroom(int(os.environ.get('GC_HEADROOM', '0')))
-import os
-eng.set_deep_lane(int(os.environ.get('DEEP_LANE', '0')))
-import os
 TIMING = os.environ.get('NO_TIMING') != '1'
 eng.set_timing(TIMING)
 prev = eng.counters()
@@ -57,13 +54,5 @@ print({n: round(float(pr[i]) / max(float(tot), 1), 3) for i, n in enumerate(name
 pt = np.zeros(16, np.uint64)
 L.lib().b200_debug_prof_tree.argtypes = [L.P, L.P]
 L.check(L.lib().b200_debug_prof_tree(eng.h, L.ptr(pt)))
-tt = float(pt[:4].sum() + pt[5])
-print('k_select_expand sampled groups', int(pt[4]), {n: round(float(pt[i]) / max(tt, 1), 3) for i, n in enumerate(['select', 'leaf_load', 'expand', 'finish+evalreq', '-', 'fused_backup']) if n != '-'}, 'mean clk/group', int(tt / max(float(pt[4]), 1)))
-if pt[11]:
-    lv = float(pt[11])
-    print('per level (B200_SELECT_PROF build, sampled groups): levels %d  row line %.0f clk | statistics %.0f clk | pick %.0f clk | total %.0f clk' % (
-        int(lv), float(pt[8]) / lv, float(pt[9]) / lv, float(pt[10]) / lv, float(pt[8] + pt[9] + pt[10]) / lv))
-if pt[15]:
-    w = float(pt[15])
-    print('path cache phase 1 (B200_SELECT_PROF build, sampled groups): walks %d  clk per walk %.0f  rounds per walk %.1f  levels served per walk %.1f | uncached levels per walk %.1f' % (
-        int(w), float(pt[12]) / w, float(pt[13]) / w, float(pt[14]) / w, float(pt[11]) / w))
+tt = float(pt[:4].sum())
+print('k_select_expand sampled groups', int(pt[4]), {n: round(float(pt[i]) / max(tt, 1), 3) for i, n in enumerate(['select', 'leaf_load', 'expand', 'finish+evalreq'])}, 'mean clk/group', int(tt / max(float(pt[4]), 1)))

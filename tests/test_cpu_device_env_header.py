@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 
-@pytest.fixture(scope="module", params=[(), ("-DB200_PLAY_UNIFIED=0",)], ids=["default", "branchy-step"])
+@pytest.fixture(scope="module", params=[()], ids=["default"])
 def host_env(request, tmp_path_factory):
     so = str(tmp_path_factory.mktemp("hostenv") / "host_env.so")
     subprocess.run(["g++", "-O2", "-shared", "-fPIC", "-x", "c++", *request.param, "-I", os.path.join(ROOT, "tetris_mcts_b200", "csrc"),
@@ -23,7 +23,7 @@ def host_env(request, tmp_path_factory):
     return C.CDLL(so)
 
 
-@pytest.mark.parametrize("env_args", [(1, 0, 0), (1, 1, 1), (2, 0, 1), (3, 1, 0)])
+@pytest.mark.parametrize("env_args", [(1, 0, 0), (1, 1, 1), (2, 0, 1), (3, 1, 0), (1, 0, 1), (1, 1, 0), (2, 1, 1), (4, 0, 0)])
 def test_device_header_steps_like_the_oracle(host_env, env_args):
     import oracle_py as O
     app, scoring, randomizer = env_args

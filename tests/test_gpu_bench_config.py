@@ -4,7 +4,8 @@ step, b200_play_move).  The C oracle agent cannot shadow 16384 games, so a sampl
 the GPU network's outputs for the same boards (the LP search is deterministic given evaluator and piece sequence, SURVEY N3), make the same
 remove_nodes() calls the head-room policy makes (agents/agent.py:246-257 driven as in tests/golden/gen_golden.py gen_agent_explicit_gc) and
 apply the same overflow_reset rule (oracle/mcts_oracle.c drop_tree).  Compared exactly: action and stats[3,7] of every move
-(agents/agent.py:153-185), the live games, and the exported arenas in the reference's array layout (agents/agent.py:58-88).
+(agents/agent.py:153-185), the live games, and the exported arenas in the reference's array layout (agents/agent.py:58-88), with the
+path cache on (the default at this configuration) and off.
 Reference loop: agents/ValueSimLP.py:44-70."""
 import numpy as np
 import pytest
@@ -18,18 +19,18 @@ def search_seed(seed, g):
     return s or 0x2545F491
 
 
-@pytest.mark.parametrize("deep_lane", [0, 164])
-def test_bench_config_sampled_games_exact(gpu_lib, oracle, deep_lane):
+@pytest.mark.parametrize("path_cache", [True, False], ids=["cache_on", "cache_off"])
+def test_bench_config_sampled_games_exact(gpu_lib, oracle, path_cache):
     from tetris_mcts_b200 import pyTetris as PT
     from tetris_mcts_b200.engine import BatchedEngine
     from tetris_mcts_b200.model.model_vv import init_weights
     n, M, sims, moves, headroom, seed = 16384, 16384, 500, 14, 16384 * 5 // 32, 123
     recs = PT.new_games(n, ARGS, np.arange(seed, seed + n, dtype=np.uint32))
     w = init_weights(0)
-    eng = BatchedEngine(n, max_nodes=M, mode="lp", eval_kind="net_tc", weights=w, seed=seed, overflow_reset=True)
+    eng = BatchedEngine(n, max_nodes=M, mode="lp", eval_kind="net_tc", weights=w, seed=seed, overflow_reset=True, path_cache=path_cache)
+    assert eng.path_cache == path_cache
     eng.set_games(recs)
     eng.set_gc_headroom(headroom)
-    eng.set_deep_lane(deep_lane)                                              # scheduling only (bench.py runs with it on)
     side = BatchedEngine(1, max_nodes=64, eval_kind="net_tc", weights=w)
 
     def cb(states):
@@ -110,39 +111,3 @@ def test_overflow_reset_rule_matches_oracle_small(gpu_lib, oracle):
             for k in ("child", "n2o", "episode", "score", "visit", "value", "variance", "obs_end", "obs_key", "game"):
                 assert np.array_equal(ex[k], want[k]), (hr, g, k)
         eng.close()
-
-
-def test_deep_lane_changes_no_result(gpu_lib):
-    """b200_set_deep_lane is scheduling only: two engines on the same games, one of them with the deepest 3 % of the games on the second stream
-    (graph path and the timed, single-stream path), give the same actions, statistics, live games and arenas for EVERY game, every move —
-    including moves with collections and dropped trees."""
-    from tetris_mcts_b200 import pyTetris as PT
-    from tetris_mcts_b200.engine import BatchedEngine
-    from tetris_mcts_b200.model.model_vv import init_weights
-    n, M, sims, moves, seed = 2048, 2048, 150, 12, 77
-    recs = PT.new_games(n, ARGS, np.arange(seed, seed + n, dtype=np.uint32))
-    w = init_weights(0)
-    engs = []
-    for lane in (0, 64, 64):
-        e = BatchedEngine(n, max_nodes=M, mode="lp", eval_kind="net_tc", weights=w, seed=seed, overflow_reset=True)
-        e.set_games(recs)
-        e.set_gc_headroom(M * 5 // 32)
-        e.set_deep_lane(lane)
-        engs.append(e)
-    engs[2].set_timing(True)
-    for mv in range(moves):
-        res = [e.play_move(sims, auto_reset=True) for e in engs]
-        for k in (1, 2):
-            assert np.array_equal(res[0][0], res[k][0]) and np.array_equal(res[0][1], res[k][1]), (mv, k)
-            assert np.array_equal(engs[0].get_games(), engs[k].get_games()), (mv, k)
-    c = [e.counters() for e in engs]
-    assert c[0]["gcs"] > 0 and c[0]["max_trace_len"] > 8
-    for key in ("sims", "expansions", "eval_requests", "gcs", "trace_levels", "new_nodes", "tree_resets"):
-        assert c[0][key] == c[1][key] == c[2][key], key
-    for g in (0, 1, 517, n - 1):
-        a, b = engs[0].export_game(g), engs[1].export_game(g)
-        assert a["root"] == b["root"]
-        for k in ("child", "n2o", "visit", "value", "variance", "score"):
-            assert np.array_equal(a[k], b[k]), (g, k)
-    for e in engs:
-        e.close()

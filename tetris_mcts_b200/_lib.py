@@ -61,7 +61,6 @@ def lib():
         L.b200_finished_games.argtypes = [P, P, C.c_int, P]
         L.b200_remove_nodes.argtypes = [P, C.c_int]
         L.b200_set_gc_headroom.argtypes = [P, C.c_int]
-        L.b200_set_deep_lane.argtypes = [P, C.c_int]
         L.b200_set_path_cache.argtypes = [P, C.c_int]
         L.b200_counters.argtypes = [P, P]
         L.b200_sync.argtypes = [P]

@@ -15,10 +15,8 @@
 #include "dist_dev.cuh"
 #include "distnet_simt.cuh"
 #include "replay_policy.cuh"
-#ifdef B200_WITH_TC
 #include "valuenet_tc.cuh"
 #include "distnet_tc.cuh"
-#endif
 
 using namespace b200;
 
@@ -69,10 +67,6 @@ struct b200_engine {
     // one simulation step captured as a CUDA graph (replayed when phase timing is off: ~7 launches + 1 memset per step, 500 steps/move)
     int gc_headroom = 0;           // b200_set_gc_headroom: collect between moves every game with fewer free slots than this
     int4 *d_pc = nullptr; int32_t *d_pc_var = nullptr, *d_pc_len = nullptr; uint4 *d_pc_sib = nullptr; int4 *d_pc_own = nullptr;   // path cache (b200_set_path_cache): allocated at the first switch-on, A.pc == nullptr while off
-    // deep lane (b200_set_deep_lane): the games with the longest traces select / collect / resume on a second stream (kernels.cuh: k_classify)
-    int deep_cap = 0; cudaStream_t stream1 = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    int32_t *d_glist0 = nullptr, *d_glist1 = nullptr, *d_nlist = nullptr, *d_nreq_deep = nullptr, *d_gc_list_deep = nullptr; uint2 *d_req_deep = nullptr;
-    int gc_pool_main = 0;          // collection scratch sets of the main k_gc launch; DEEP_GC_BLOCKS more follow for the deep lane's
     cudaGraphExec_t step_exec = nullptr; bool step_graph_failed = false;
     uint64_t step_launches[PH_N] = {0};
 };
@@ -83,7 +77,8 @@ static void drop_step_graph(b200_engine *e) {
     e->step_graph_failed = false;
 }
 
-constexpr int DEEP_GC_BLOCKS = 8;
+static inline int blocks_groups(int G) { return (G + GROUPS_PER_BLOCK - 1) / GROUPS_PER_BLOCK; }
+static inline int gc_blocks(const b200_engine *e) { int b = e->n_sm * 4; return e->A.G < b ? e->A.G : b; }   // k_gc CTAs (one scratch set each)
 
 // k_backup's per-warp bitmap of the trace's observations (path cache on): max_nodes bits, four warps per CTA
 static inline int backup_bitmap_words(const Arena &A) { return A.pc ? (A.M + 31) / 32 : 0; }
@@ -213,12 +208,11 @@ extern "C" int b200_engine_create(const b200_config *cfg, b200_engine **out) {
     rc |= dalloc(e, &A.trace, G * A.trace_max); rc |= dalloc(e, &A.trace_len, G); rc |= dalloc(e, &A.leaf_kind, G);
     rc |= dalloc(e, &A.trace_meta, G * A.trace_max);
     {   // collection scratch: one set per k_gc CTA (gc_blocks), not per game
-        e->gc_pool_main = e->n_sm * 4 < A.G ? e->n_sm * 4 : A.G;
-        const size_t pool = (size_t)(e->gc_pool_main + DEEP_GC_BLOCKS) * A.M;
+        const size_t pool = (size_t)gc_blocks(e) * A.M;
         rc |= dalloc(e, &A.nmark, pool); rc |= dalloc(e, &A.omark, pool); rc |= dalloc(e, &A.gc_queue, pool * 2);
     }
     rc |= dalloc(e, &A.cur, G * REC_WORDS);
-    rc |= dalloc(e, &A.req, G * 8); rc |= dalloc(e, &A.n_req, 4);
+    rc |= dalloc(e, &A.req, G * 8); rc |= dalloc(e, &A.n_req, 2);
     rc |= dalloc(e, &A.gc_list, G); rc |= dalloc(e, &A.pending, G); rc |= dalloc(e, &A.resume_a, G);
     rc |= dalloc(e, &A.eval_out, G * 8); rc |= dalloc(e, &A.rollout_val, G);
     rc |= dalloc(e, &A.counters, 48);
@@ -258,15 +252,11 @@ extern "C" int b200_engine_destroy(b200_engine *e) {
     if (!e) return B200_OK;
     if (e->stream) cudaStreamSynchronize(e->stream);
     if (e->step_exec) cudaGraphExecDestroy(e->step_exec);
-#ifdef B200_WITH_TC
     tc_destroy(e->tc_state);
     dn_tc_destroy(e->dn_tc_state);
-#endif
     for (void *p : e->allocs) cudaFree(p);
     for (auto &ev : e->ev) cudaEventDestroy(ev);
     if (e->t0) { cudaEventDestroy(e->t0); cudaEventDestroy(e->t1); }
-    if (e->stream1) cudaStreamDestroy(e->stream1);
-    if (e->ev_fork) { cudaEventDestroy(e->ev_fork); cudaEventDestroy(e->ev_join); }
     if (e->stream && e->own_stream) cudaStreamDestroy(e->stream);
     delete e;
     return B200_OK;
@@ -279,7 +269,6 @@ extern "C" int b200_engine_set_stream(b200_engine *e, void *cuda_stream) {
     if (!e) return fail(B200_ERR_BAD_ARG, "null engine");
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaStreamSynchronize(e->stream));
-    if (e->stream1) CK(cudaStreamSynchronize(e->stream1));
     drop_step_graph(e);
     cudaStream_t ns = (cudaStream_t)cuda_stream;
     const bool own = ns == nullptr;
@@ -336,12 +325,10 @@ extern "C" int b200_load_weights(b200_engine *e, const float *w) {
     e->W.wfc1 = e->W.b1 + 96; e->W.bfc1 = e->W.wfc1 + (size_t)1792 * 256; e->W.wout = e->W.bfc1 + 256;
     e->W.bout = e->W.wout + 512; e->W.ub = e->W.bout + 2; e->W.lb = e->W.bout + 4;
     CK(cudaFuncSetAttribute(k_vn_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, VN_SMEM_BYTES));
-#ifdef B200_WITH_TC
     {
         int rc = tc_prepare(&e->tc_state, w, e->stream);
         if (rc) return fail(B200_ERR_CUDA, "tensor-core weight preparation failed");
     }
-#endif
     e->have_weights = true;
     drop_step_graph(e);
     return B200_OK;
@@ -359,7 +346,6 @@ static int ensure_act3(b200_engine *e, size_t rows) {
 static int launch_net(b200_engine *e, const uint2 *req, const int32_t *n_req, const uint32_t *keys, int M, float2 *eval_out,
                       size_t max_rows) {
     if (!e->have_weights) return fail(B200_ERR_NO_WEIGHTS, "b200_load_weights was not called");
-#ifdef B200_WITH_TC
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
         TcState *st = (TcState *)e->tc_state;
         const uint8_t *act3_before = st->d_act3;
@@ -367,7 +353,7 @@ static int launch_net(b200_engine *e, const uint2 *req, const int32_t *n_req, co
         if (act3_before && st->d_act3 != act3_before) drop_step_graph(e);   // a larger standalone batch moved the activation buffer
         {
             PhaseTimer t(e, PH_CONV);
-            k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, e->stream>>>(e->W, st->TW, req, n_req, nullptr, keys, M, st->d_act3, (int)st->tiles,
+            k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, e->stream>>>(e->W, st->TW, req, n_req, keys, M, st->d_act3, (int)st->tiles,
                                                                     e->timing ? e->A.counters + 16 : nullptr);
         }
         {
@@ -377,7 +363,6 @@ static int launch_net(b200_engine *e, const uint2 *req, const int32_t *n_req, co
         CK(cudaGetLastError());
         return B200_OK;
     }
-#endif
     {
         const float *act3_before = e->d_act3;
         if (ensure_act3(e, max_rows)) return B200_ERR_CUDA;
@@ -410,9 +395,7 @@ extern "C" int b200_load_dist_weights(b200_engine *e, const float *w, int atoms)
     e->DW = dn_pointers(e->d_dnw, atoms);
     CK(cudaFuncSetAttribute(k_dn_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, DN_CONV_SMEM));
     CK(cudaFuncSetAttribute(k_dn_fc, cudaFuncAttributeMaxDynamicSharedMemorySize, DN_FC_SMEM));
-#ifdef B200_WITH_TC
     if (dn_tc_prepare(&e->dn_tc_state, w, atoms, e->stream)) return fail(B200_ERR_CUDA, "tensor-core weight preparation (distributional network) failed");
-#endif
     e->have_dist_weights = true;
     drop_step_graph(e);
     return B200_OK;
@@ -420,7 +403,6 @@ extern "C" int b200_load_dist_weights(b200_engine *e, const float *w, int atoms)
 
 static int launch_distnet_on(b200_engine *e, const uint2 *req, const int32_t *n_req, const uint32_t *keys, int M, float *out, size_t max_rows) {
     if (!e->have_dist_weights) return fail(B200_ERR_NO_WEIGHTS, "b200_load_dist_weights was not called");
-#ifdef B200_WITH_TC
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
         DnTcState *st = (DnTcState *)e->dn_tc_state;
         bool moved = false;
@@ -437,7 +419,6 @@ static int launch_distnet_on(b200_engine *e, const uint2 *req, const int32_t *n_
         CK(cudaGetLastError());
         return B200_OK;
     }
-#endif
     if (e->dn_rows < max_rows) {
         const bool had = e->d_dn_act != nullptr;
         if (had) { cudaStreamSynchronize(e->stream); dfree(e, e->d_dn_act); e->d_dn_act = nullptr; e->dn_rows = 0; }
@@ -483,8 +464,6 @@ extern "C" int b200_distnet_forward(b200_engine *e, const int8_t *states, int k,
 }
 
 // ---------------------------------------------------------------------------------------------------- games / roots
-static inline int blocks_groups(int G) { return (G + GROUPS_PER_BLOCK - 1) / GROUPS_PER_BLOCK; }
-static inline int gc_blocks(b200_engine *e) { int b = e->n_sm * 4; return e->A.G < b ? e->A.G : b; }
 
 static int check_status(b200_engine *e) {   // cheap: max over the status array computed on the host after a small copy
     std::vector<int32_t> st(e->A.G);
@@ -525,7 +504,6 @@ extern "C" int b200_set_path_cache(b200_engine *e, int on) {
     if (on) {
         if (e->A.mode != MODE_LP) return fail(B200_ERR_BAD_ARG, "the path cache serves B200_MODE_LP (its coherence rules rest on the LP backup)");
         if (e->A.M > PC_MAX_NODES) return fail(B200_ERR_BAD_ARG, "the path cache needs max_nodes <= 65536 (k_backup's bitmap of the trace's observations)");
-        if (B200_FUSED_BACKUP) return fail(B200_ERR_BAD_ARG, "the path cache needs the separate k_backup launch (B200_FUSED_BACKUP=0)");
     }
     CK(cudaStreamSynchronize(e->stream));
     drop_step_graph(e);
@@ -540,30 +518,6 @@ extern "C" int b200_set_path_cache(b200_engine *e, int on) {
     e->A.pc_len = on ? e->d_pc_len : nullptr;
     e->A.pc_sib = on ? e->d_pc_sib : nullptr;
     e->A.pc_own = on ? e->d_pc_own : nullptr;
-    return B200_OK;
-}
-
-extern "C" int b200_set_deep_lane(b200_engine *e, int max_games) {
-    if (!e || max_games < 0 || max_games > e->A.G) return fail(B200_ERR_BAD_ARG, "0 <= max_games <= n_games");
-    CK(cudaSetDevice(e->cfg.device));
-    drop_step_graph(e);
-    if (max_games > 0) {
-        if (!e->stream1) {
-            int lo = 0, hi = 0;
-            CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-            CK(cudaStreamCreateWithPriority(&e->stream1, cudaStreamNonBlocking, hi));      // the few deep CTAs go first wherever a slot frees up
-            CK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming));
-            if (dalloc(e, &e->d_glist0, (size_t)e->A.G) || dalloc(e, &e->d_nlist, 2) || dalloc(e, &e->d_nreq_deep, 2)) return B200_ERR_CUDA;
-        }
-        CK(cudaStreamSynchronize(e->stream));
-        dfree(e, e->d_glist1); dfree(e, e->d_gc_list_deep); dfree(e, e->d_req_deep);
-        e->d_glist1 = nullptr; e->d_gc_list_deep = nullptr; e->d_req_deep = nullptr;
-        if (dalloc(e, &e->d_glist1, (size_t)max_games) || dalloc(e, &e->d_gc_list_deep, (size_t)max_games) || dalloc(e, &e->d_req_deep, (size_t)max_games * 8))
-            return B200_ERR_CUDA;
-        CK(cudaStreamSynchronize(e->stream));
-    }
-    e->deep_cap = max_games;
     return B200_OK;
 }
 
@@ -605,81 +559,10 @@ extern "C" int b200_get_games(b200_engine *e, uint32_t *recs) {
 }
 
 // ---------------------------------------------------------------------------------------------------- simulations
-static bool deep_lane_on(const b200_engine *e) {
-#ifdef B200_WITH_TC
-    return e->deep_cap > 0 && (e->A.mode == MODE_LP || e->A.mode == MODE_SINGLE) && e->cfg.eval_kind == B200_EVAL_NET_TC && !B200_FUSED_BACKUP;
-#else
-    return false;
-#endif
-}
-
-#ifdef B200_WITH_TC
-// The step with the deep lane: the deepest games (k_classify, once per move) walk on stream1 while the others walk, collect AND run their
-// network launch on the engine's stream; the lanes join, the deep lane's requests go behind the others' (k_merge_requests), a second, small
-// k_tc_conv evaluates them, and k_tc_fc / k_backup work on all of them as before.  With phase timing on everything runs on one stream
-// in the same order.  Which lane a game is in changes nothing in its results.
-static int enqueue_step_lanes(b200_engine *e) {
-    const Arena &A = e->A;
-    const int G = A.G;
-    if (!e->have_weights) return fail(B200_ERR_NO_WEIGHTS, "b200_load_weights was not called");
-    TcState *st = (TcState *)e->tc_state;
-    const uint8_t *act3_before = st->d_act3;
-    if (tc_ensure_act3(st, (size_t)G * (A.mode == MODE_LP ? 7 : 1), e->stream)) return fail(B200_ERR_CUDA, "act3 (tensor-core layout) allocation failed");
-    if (act3_before && st->d_act3 != act3_before) drop_step_graph(e);
-    cudaStream_t s0 = e->stream, s1 = e->timing ? e->stream : e->stream1;
-    Arena A0 = A, A1 = A;
-    A0.glist = e->d_glist0; A0.n_list = e->d_nlist;
-    A1.glist = e->d_glist1; A1.n_list = e->d_nlist + 1;
-    A1.req = e->d_req_deep; A1.n_req = e->d_nreq_deep; A1.gc_list = e->d_gc_list_deep;
-    A1.nmark += (size_t)e->gc_pool_main * A.M; A1.omark += (size_t)e->gc_pool_main * A.M; A1.gc_queue += (size_t)e->gc_pool_main * A.M * 2;
-    A0.prof = e->timing ? A.counters + 32 : nullptr;
-    CK(cudaMemsetAsync(A.n_req, 0, 4 * sizeof(int32_t), s0));
-    CK(cudaMemsetAsync(e->d_nreq_deep, 0, 2 * sizeof(int32_t), s0));
-    if (s1 != s0) { CK(cudaEventRecord(e->ev_fork, s0)); CK(cudaStreamWaitEvent(s1, e->ev_fork, 0)); }
-    const int deep_groups = blocks_groups(e->deep_cap);
-    {
-        PhaseTimer t(e, PH_SELECT);
-        k_select_expand<<<(G + SE_GAMES_PER_BLOCK - 1) / SE_GAMES_PER_BLOCK, TPB, 0, s0>>>(A0);
-        k_select_expand<<<(e->deep_cap + SE_GAMES_PER_BLOCK - 1) / SE_GAMES_PER_BLOCK, TPB, 0, s1>>>(A1);
-    }
-    {
-        PhaseTimer t(e, PH_GC);
-        k_gc<<<gc_blocks(e), GC_THREADS, 0, s0>>>(A0);
-        k_expand_resume<<<blocks_groups(G), TPB, 0, s0>>>(A0);
-        k_gc<<<DEEP_GC_BLOCKS, GC_THREADS, 0, s1>>>(A1);
-        k_expand_resume<<<deep_groups, TPB, 0, s1>>>(A1);
-    }
-    {
-        PhaseTimer t(e, PH_CONV);
-        k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, s0>>>(e->W, st->TW, A.req, A.n_req, nullptr, A.key, A.M, st->d_act3, (int)st->tiles,
-                                                          e->timing ? A.counters + 16 : nullptr);
-    }
-    if (s1 != s0) { CK(cudaEventRecord(e->ev_join, s1)); CK(cudaStreamWaitEvent(s0, e->ev_join, 0)); }
-    {
-        PhaseTimer t(e, PH_CONV);
-        k_merge_requests<<<1, 256, 0, s0>>>(A.req, A.n_req, e->d_req_deep, e->d_nreq_deep);
-        k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, s0>>>(e->W, st->TW, A.req, A.n_req, A.n_req + 2, A.key, A.M, st->d_act3, (int)st->tiles, nullptr);
-    }
-    {
-        PhaseTimer t(e, PH_FC);
-        k_tc_fc<<<e->n_sm, TCF_THREADS, TCF_SMEM, s0>>>(e->W, st->TW, st->d_act3, (int)st->tiles, A.req, A.n_req, A.eval_out);
-    }
-    {
-        PhaseTimer t(e, PH_BACKUP);
-        k_backup<<<(G + 3) / 4, 128, backup_smem(A), s0>>>(A, backup_bitmap_words(A));
-    }
-    CK(cudaGetLastError());
-    return B200_OK;
-}
-#endif
-
 // One simulation step of every game: select+expand -> (collect garbage, resume) -> evaluate -> backup.
 static int enqueue_step(b200_engine *e) {
     const Arena &A = e->A;
     const int G = A.G;
-#ifdef B200_WITH_TC
-    if (deep_lane_on(e)) return enqueue_step_lanes(e);
-#endif
     CK(cudaMemsetAsync(A.n_req, 0, 2 * sizeof(int32_t), e->stream));
     {
         PhaseTimer t(e, PH_SELECT);
@@ -710,7 +593,7 @@ static int enqueue_step(b200_engine *e) {
         int rc = launch_net(e, A.req, A.n_req, A.key, A.M, A.eval_out, (size_t)G * (A.mode == MODE_LP ? 7 : 1));
         if (rc) return rc;
     }
-    if (A.mode == MODE_DIST || !B200_FUSED_BACKUP) {   // otherwise the next k_select_expand (or run_sims' final k_backup) folds this step's traces
+    {
         PhaseTimer t(e, PH_BACKUP);
         if (A.mode == MODE_DIST) k_dist_backup<<<(G + 3) / 4, 128, 0, e->stream>>>(A);
         else k_backup<<<(G + 3) / 4, 128, backup_smem(A), e->stream>>>(A, backup_bitmap_words(A));
@@ -744,8 +627,6 @@ extern "C" int b200_run_sims(b200_engine *e, int sims) {
     const bool need_net = A.mode != MODE_VANILLA && e->cfg.eval_kind != B200_EVAL_SYNTHETIC;
     if (need_net && !(A.mode == MODE_DIST ? e->have_dist_weights : e->have_weights)) return fail(B200_ERR_NO_WEIGHTS, "b200_load_weights was not called");
     CK(cudaMemsetAsync(A.counters + 12, 0, sizeof(unsigned long long), e->stream));   // counter 12: the longest trace of this call
-    if (deep_lane_on(e) && sims > 0)     // this move's lanes, from the trace lengths of the previous move's last simulation
-        k_classify<<<1, 1024, 0, e->stream>>>(A, e->deep_cap, e->d_glist0, e->d_nlist, e->d_glist1, e->d_nlist + 1);
     for (int s = 0; s < sims; ++s) {
         if (!e->timing && e->step_exec) {
             CK(cudaGraphLaunch(e->step_exec, e->stream));
@@ -755,10 +636,6 @@ extern "C" int b200_run_sims(b200_engine *e, int sims) {
         int rc = enqueue_step(e);
         if (rc) return rc;
         if (!e->timing && !e->step_exec && !e->step_graph_failed) capture_step(e);
-    }
-    if (B200_FUSED_BACKUP && A.mode != MODE_DIST && sims > 0) {   // the last simulation's traces (the others were folded by the next step's k_select_expand)
-        PhaseTimer t(e, PH_BACKUP);
-        k_backup<<<(A.G + 3) / 4, 128, backup_smem(A), e->stream>>>(A, backup_bitmap_words(A));
     }
     CK(cudaGetLastError());
     return B200_OK;
@@ -845,7 +722,7 @@ extern "C" int b200_debug_prof(b200_engine *e, uint64_t *out16) {   // clock64 p
     return B200_OK;
 }
 
-extern "C" int b200_debug_prof_tree(b200_engine *e, uint64_t *out16) {   // clock64 sums of sampled groups of k_select_expand (timing mode); 8..11: per-level split (B200_SELECT_PROF builds)
+extern "C" int b200_debug_prof_tree(b200_engine *e, uint64_t *out16) {   // clock64 sums of sampled groups of k_select_expand (timing mode)
     if (!e || !out16) return fail(B200_ERR_BAD_ARG, "null argument");
     CK(cudaSetDevice(e->cfg.device));
     CK(cudaMemcpyAsync(out16, e->A.counters + 32, 16 * 8, cudaMemcpyDeviceToHost, e->stream));
@@ -1001,7 +878,6 @@ extern "C" int b200_debug_act3(b200_engine *e, const int8_t *states, int k, floa
     std::vector<float> v(k), var(k);
     int rc = b200_valuenet_forward(e, states, k, v.data(), var.data());   // leaves act3 of these k boards in the scratch buffers
     if (rc) return rc;
-#ifdef B200_WITH_TC
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
         TcState *st = (TcState *)e->tc_state;
         size_t bytes = (size_t)2 * st->tiles * ACT3_KCHUNKS * 2048;
@@ -1020,7 +896,6 @@ extern "C" int b200_debug_act3(b200_engine *e, const int8_t *states, int k, floa
             }
         return B200_OK;
     }
-#endif
     std::vector<float> h((size_t)k * 1792);
     CK(cudaMemcpy(h.data(), e->d_act3, h.size() * 4, cudaMemcpyDeviceToHost));
     for (int r = 0; r < k; ++r)

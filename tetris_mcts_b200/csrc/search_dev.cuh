@@ -28,10 +28,6 @@ constexpr int ZTABLE_N = 65536;   // z(n) table computed on the host with the re
 
 enum : int { ST_OK = 0, ST_ARENA_FULL = 1, ST_TRACE_FULL = 2, ST_NEED_GC = 3, ST_RESET_DONE = 4 };   // RESET_DONE: k_gc dropped the tree (overflow_reset), only the re-rooting is left
 enum : int { LEAF_TERMINAL = 0, LEAF_EXPANDED = 1, LEAF_SUSPENDED = 2, LEAF_DONE = 3 };   // DONE: the trace has been backed up
-#ifndef B200_FUSED_BACKUP
-#define B200_FUSED_BACKUP 0   // 1: the backup of a game's previous simulation runs at the start of k_select_expand (kernels.cuh: backup_game);
-                              // exact (59 GPU tests) but measured 4 % slower than the separate warp-per-game k_backup on B200, so off
-#endif
 enum : int { PEND_NONE = 0, PEND_EXPAND = 1, PEND_ROOT = 2 };
 enum : int { MODE_LP = 0, MODE_SINGLE = 1, MODE_VANILLA = 2, MODE_DIST = 3 };
 constexpr int NSTAT_WORDS = 8;    // node_stats row: {visit, mean, reward, variance, M2, -, -, -} (agents/core_distributional.py:109-124)
@@ -77,8 +73,6 @@ struct Arena {
     float *rollout_val;            // [G]
     // distributional mode (agents/core_distributional.py; BASELINE config 5): node-indexed statistics and value histograms
     float *nstat; float *ndist; float *dist_eval; int dist_bins; double dist_vmin, dist_vmax;   // [G][M][8], [G][M][bins], [G][bins]
-    // lanes (b200_set_deep_lane): the select / collect / resume kernels of a lane work on the games glist[0 .. *n_list); nullptr: every game
-    const int32_t *glist; const int32_t *n_list;
     unsigned long long *counters;  // [8] 0 sims 1 expansions 2 eval requests 3 gcs 4 trace levels 5 rollout steps 6 new nodes
     unsigned long long *prof;      // timing mode only: clock64 sums of k_select_expand {select, leaf load, expand, finish, groups sampled}
 };
@@ -113,11 +107,6 @@ struct GrpW {
 };
 
 __device__ __forceinline__ size_t node_at(const Arena &A, int g, int i) { return (size_t)g * A.M + i; }
-// the game that slot `slot` of a lane's k_select_expand works on (A.G = none)
-__device__ __forceinline__ int lane_game(const Arena &A, int slot) {
-    if (!A.glist) return slot < A.G ? slot : A.G;
-    return slot < *A.n_list ? A.glist[slot] : A.G;
-}
 
 // ------------------------------------------------------------------ exact arithmetic (see header comment)
 __device__ __forceinline__ float ztab(const Arena &A, int n) {
@@ -193,35 +182,16 @@ __device__ __forceinline__ uint32_t link_word(const Uniq &u) {
 }
 
 // ------------------------------------------------------------------ cache-warming loads (see warm_expand)
-#ifndef B200_WARM_EXPAND
-#define B200_WARM_EXPAND 1
-#endif
-#ifndef B200_WARM_SELECT
-#define B200_WARM_SELECT 0   // round 1 (moves 0-3, shallow trees): -1 % on k_select_expand; round 2 (moves 0-5, mean depth 36-62): +13 % -> off
-#endif
 // L2 residency hints (performance only).  One simulation step streams ~200 MB of activations (conv -> fc) and ~20 MB of new
 // nodes through the 126 MB L2, so without hints nothing of the trees survives from one step to the next although every step
-// re-walks the same top levels.  The first B200_L2_HOT_LEVELS levels of every game's walk (row line + statistics, ~3.7 MB per
-// level at 16384 games) are loaded / stored with an evict_last policy, the activation stream with evict_first.
-#ifndef B200_L2_HOT_LEVELS
-#define B200_L2_HOT_LEVELS 16
-#endif
-#ifndef B200_ROLL_PREFETCH
-#define B200_ROLL_PREFETCH 0   // 1: rolling L2 prefetch along the previous simulation's trace inside the walk (select_trace)
-#endif
-#ifndef B200_ROW_HINT
-#define B200_ROW_HINT 1        // 0: the walk loads its row words without an L2 policy (the statistics keep theirs)
-#endif
+// re-walks the same top levels.  The first L2_HOT_LEVELS levels of every game's walk (row line + statistics, ~3.7 MB per
+// level at 16384 games) are loaded / stored with an evict_last policy.
+constexpr int L2_HOT_LEVELS = 16;
 __device__ __forceinline__ uint64_t l2_policy(bool keep) {
     uint64_t last, normal;
     asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(last));
     asm("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(normal));
     return keep ? last : normal;
-}
-__device__ __forceinline__ uint64_t l2_policy_stream() {
-    uint64_t p;
-    asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-    return p;
 }
 __device__ __forceinline__ int32_t ldg_hint(const int32_t *p, uint64_t pol) {
     int32_t v;
@@ -378,53 +348,25 @@ struct ArenaAcc {
         s = 0.f; lw = 0u;
         o = 0;
         if (on) {
-#if B200_L2_HOT_LEVELS > 0 && B200_ROW_HINT
-            const uint64_t pol = l2_policy(depth < B200_L2_HOT_LEVELS);
+            const uint64_t pol = l2_policy(depth < L2_HOT_LEVELS);
             o = ldg_hint(row + 8, pol);
             s = __int_as_float(ldg_hint(row + 16, pol));
             lw = (uint32_t)ldg_hint(row + 24, pol);
-#else
-            o = row[8];
-            s = __int_as_float(row[16]);
-            lw = (uint32_t)row[24];
-#endif
         }
         s_idx = gp.bcast(s, 7);
         u.is_first = lw >> 31; u.rep_lane = (int)((lw >> 28) & 7u); u.rep_c = (int)(lw & LINK_NODE_MASK);
         u.rep_s = gp.bcast(s, u.rep_lane);
         u.first_mask = gp.ballot(u.is_first);
-#if B200_WARM_SELECT
-        if (on && u.is_first) {   // start fetching every candidate child's row while the statistics are loaded and compared
-            const int32_t *cr = rowg + (size_t)u.rep_c * ROW_WORDS;
-            touch32(cr + 8); touch32(cr + 16); touch32(cr + 24);
-        }
-#endif
     }
     __device__ __forceinline__ int4 stat(int o) const { return statg[o]; }
     __device__ __forceinline__ void set_stat(int o, int4 st) const { statg[o] = st; }
-    // the same, for a node at `depth` of the current walk (see B200_L2_HOT_LEVELS)
-    __device__ __forceinline__ int4 stat(int o, int depth) const {
-#if B200_L2_HOT_LEVELS > 0
-        return ldg_hint(statg + o, l2_policy(depth < B200_L2_HOT_LEVELS));
-#else
-        return statg[o];
-#endif
-    }
-    __device__ __forceinline__ void set_stat(int o, int4 st, int depth) const {
-#if B200_L2_HOT_LEVELS > 0
-        stg_hint(statg + o, st, l2_policy(depth < B200_L2_HOT_LEVELS));
-#else
-        statg[o] = st;
-#endif
-    }
+    // the same, for a node at `depth` of the current walk (see L2_HOT_LEVELS)
+    __device__ __forceinline__ int4 stat(int o, int depth) const { return ldg_hint(statg + o, l2_policy(depth < L2_HOT_LEVELS)); }
+    __device__ __forceinline__ void set_stat(int o, int4 st, int depth) const { stg_hint(statg + o, st, l2_policy(depth < L2_HOT_LEVELS)); }
     __device__ __forceinline__ void meta(int idx, int depth, int &o, float &s) const {
         const int32_t *row = rowg + (size_t)idx * ROW_WORDS;
-#if B200_L2_HOT_LEVELS > 0
-        const uint64_t pol = l2_policy(depth < B200_L2_HOT_LEVELS);
+        const uint64_t pol = l2_policy(depth < L2_HOT_LEVELS);
         o = ldg_hint(row + 15, pol); s = __int_as_float(ldg_hint(row + 23, pol));
-#else
-        o = row[15]; s = __int_as_float(row[23]);
-#endif
     }
     __device__ __forceinline__ void put_trace(int d, int idx) const { traceg[d] = idx; }
     __device__ __forceinline__ int get_trace(int d) const { return traceg[d]; }
@@ -433,18 +375,6 @@ struct ArenaAcc {
     __device__ __forceinline__ void get_trace_meta_raw(int d, int &oraw, float &s) const { const int2 m = tmetag[d]; oraw = m.x; s = __int_as_float(m.y); }   // with the pick in bits 28-30
     __device__ __forceinline__ uint32_t rand() const { uint32_t sr = A.srng[g]; uint32_t r = rng_next(sr); A.srng[g] = sr; return r; }
     __device__ __forceinline__ float z(int n) const { return (zs && n >= 0 && n < ZS_N) ? zs[n] : ztab(A, n); }
-    __device__ __forceinline__ unsigned long long *level_prof() const { return (A.prof && (g & 63) == 0) ? A.prof + 8 : nullptr; }
-    // rolling prefetch along the PREVIOUS simulation's trace (B200_ROLL_PREFETCH): its length, one of its levels, and the L2 requests for a level
-    __device__ __forceinline__ int prev_trace_len() const { return A.trace_len[g]; }
-    __device__ __forceinline__ void prev_trace(int lv, int &idx, int &o) const { idx = traceg[lv]; o = tmetag[lv].x & (int)TMETA_OBS_MASK; }
-    __device__ __forceinline__ void prefetch_level(int idx, int o) const {
-        const char *r = reinterpret_cast<const char *>(rowg + (size_t)idx * ROW_WORDS);
-        prefetch_l2(r + 32); prefetch_l2(r + 96);                                     // the walk reads words 8..31 of the row line
-        const char *st = reinterpret_cast<const char *>(statg + o);                   // siblings' observation ids are consecutive (free-list pops):
-        const char *lo = reinterpret_cast<const char *>(statg), *hi = lo + (size_t)A.M * sizeof(int4) - 1;   // their statistics surround the chosen one's
-        const char *a = st - 64, *b = st + 64;
-        prefetch_l2(st); prefetch_l2(a < lo ? lo : a); prefetch_l2(b > hi ? hi : b);
-    }
 };
 
 struct RefAcc {   // child int32[M,7], visit int32[M], value/variance/score f32[M], n_to_o int32[M]  (core.cpp:20-26)
@@ -477,17 +407,10 @@ struct RefAcc {   // child int32[M,7], visit int32[M], value/variance/score f32[
     __device__ __forceinline__ void put_trace_meta(int, int, float) const {}
     __device__ __forceinline__ uint32_t rand() const { uint32_t sr = *rng; uint32_t r = rng_next(sr); *rng = sr; return r; }
     __device__ __forceinline__ float z(int n) const { return ztab(*A, n); }
-    __device__ __forceinline__ unsigned long long *level_prof() const { return nullptr; }
-    __device__ __forceinline__ int prev_trace_len() const { return 0; }
-    __device__ __forceinline__ void prev_trace(int, int &idx, int &o) const { idx = 0; o = 0; }
-    __device__ __forceinline__ void prefetch_level(int, int) const {}
 };
 
 // ------------------------------------------------------------------ select (core.h:167-224)
 // Returns the leaf; writes the trace.  All 8 lanes return the same values.
-#ifndef B200_SELECT_PROF
-#define B200_SELECT_PROF 0   // development aid: clock64 split of one walk level (row line landed | statistics landed | child picked), sampled groups
-#endif
 // Warp-lockstep walk: the four 8-lane groups of a warp descend their four trees level by level TOGETHER, all 32 lanes converged, so
 // that every shuffle and vote carries the literal full mask (GrpW).  `active` = this lane's group has a tree to walk; a group that
 // has reached its leaf idles (predicated) until the deepest of the four is done.  Returns the leaf; writes the trace; all 8 lanes of
@@ -497,23 +420,6 @@ __device__ __forceinline__ int select_trace(const Acc &acc, bool active, int roo
     const GrpW gp;
     int idx = root, D = 0;
     bool walking = active;
-#if B200_ROLL_PREFETCH
-    // A game's walk mostly retraces its previous simulation's path, and every level is two DEPENDENT misses.  The previous trace is known
-    // (trace / trace_meta are overwritten level by level as this walk advances), so lanes 0..3 of a group request, every four levels, the row
-    // lines and statistics lines of the old path's levels +2..+5 from L2: where the new walk follows the old path it finds them there.  A
-    // short look-ahead keeps the footprint at ~16 MB for 16384 games (requesting the whole old path before the walk — B200_PV_PREFETCH —
-    // is 277 MB per step against a 126 MB L2 and was slower).  The old entries are loaded one batch earlier than they are used.
-    const int prev_len = active ? acc.prev_trace_len() : 0;
-    int pf_idx = 0, pf_o = 0, it = 0;
-    if (gp.lane < 4 && 2 + gp.lane < prev_len) acc.prev_trace(2 + gp.lane, pf_idx, pf_o);
-#endif
-#if B200_SELECT_PROF
-    unsigned long long *lp = (active && gp.lane == 0) ? acc.level_prof() : nullptr;
-    long long lt = lp ? clock64() : 0;
-#define LEVEL_PROF(i) do { if (lp && walking) { const long long _n = clock64(); atomicAdd(&lp[i], (unsigned long long)(_n - lt)); lt = _n; } } while (0)
-#else
-#define LEVEL_PROF(i) do { } while (0)
-#endif
     // core.h:65-105 for one level, from the values every lane holds for its child slot (`on`: this lane's group is at a node WITH children):
     // check_low, then policy_clt.  Shared by the cached and the uncached form of a level, so both pick bit for bit the same child.
     auto choose = [&](bool on, const Uniq &u, const int4 &st, float s_idx, float &val_out, float &root_out) -> int {
@@ -561,14 +467,7 @@ __device__ __forceinline__ int select_trace(const Acc &acc, bool active, int roo
         const int pcl = (walking && acc.pcg) ? acc.pc_len : 0;          // group-uniform
         bool fast = pcl > 0;
         int n_cached = 0;
-#if B200_SELECT_PROF
-        const long long p1t = clock64();
-        int p1_rounds = 0;
-#endif
         while (__any_sync(0xffffffffu, fast)) {
-#if B200_SELECT_PROF
-            ++p1_rounds;
-#endif
             const int L = D + gp.lane;                                  // this lane's level
             const bool have = fast && L < pcl;
             int e_node = 0, e_own = 0, pick_prev = 7, pick = 7, next = 0; float s_idx = 0.f;
@@ -606,22 +505,10 @@ __device__ __forceinline__ int select_trace(const Acc &acc, bool active, int roo
             }
         }
         if (cached_levels) *cached_levels = n_cached;
-#if B200_SELECT_PROF
-        if (lp) { lt = clock64(); atomicAdd(&lp[4], (unsigned long long)(lt - p1t)); atomicAdd(&lp[5], (unsigned long long)p1_rounds); atomicAdd(&lp[6], (unsigned long long)n_cached); atomicAdd(&lp[7], 1ull); }
-#endif
     }
     // ---- phase 2: uncached levels (two dependent random accesses each); with the path cache on, each of them leaves its entry behind
     while (__any_sync(0xffffffffu, walking)) {
         if (walking && D >= trace_max) { status = ST_TRACE_FULL; walking = false; }
-#if B200_ROLL_PREFETCH
-        if ((it & 3) == 0) {                                             // (warp-uniform: the walking groups of a warp are at the same level)
-            if (walking && pf_idx > 0) acc.prefetch_level(pf_idx, pf_o);
-            pf_idx = 0;
-            const int lv = it + 6 + gp.lane;
-            if (walking && gp.lane < 4 && lv < prev_len) acc.prev_trace(lv, pf_idx, pf_o);
-        }
-        ++it;
-#endif
         if (walking) {
             if (gp.lane == 0) acc.put_trace(D, idx);
             ++D;
@@ -630,11 +517,9 @@ __device__ __forceinline__ int select_trace(const Acc &acc, bool active, int roo
         int o; float s_idx, s_own; uint32_t lw;
         Uniq u;
         acc.level(gp, walking, idx, D - 1, o, s_idx, u, s_own, lw);
-        LEVEL_PROF(0);
         if (u.first_mask == 0) walking = false;                         // core.h:200 no children: leaf (group-uniform)
         int4 st = make_int4(0, 0, 0, 0);
         if (walking && u.is_first) st = acc.stat(o, D);                 // the children live one level below
-        LEVEL_PROF(1);
         float q_val, q_root;
         const int pick = choose(walking, u, st, s_idx, q_val, q_root);
         const int next = gp.bcast(u.rep_c, pick);
@@ -647,12 +532,7 @@ __device__ __forceinline__ int select_trace(const Acc &acc, bool active, int roo
             }
         }
         if (walking) idx = next;
-        LEVEL_PROF(2);
-#if B200_SELECT_PROF
-        if (lp && walking) atomicAdd(&lp[3], 1ull);
-#endif
     }
-#undef LEVEL_PROF
     __syncwarp();
     D_out = D;
     return idx;
@@ -854,7 +734,6 @@ __device__ __noinline__ void reset_tree(const Arena &A, const Grp &gp, int g, in
 // table slots, then (on a hash match) the candidate record / row / key; lane 7 touches the counters and the free-list tails.  The
 // ordered loop then runs on L1/L2 hits.  Real loads (volatile asm) are used: a prefetch instruction may be dropped.
 __device__ __forceinline__ void warm_expand(const Arena &A, const Grp &gp, int g, uint32_t h, uint32_t hk) {
-#if B200_WARM_EXPAND
     const int M = A.M, H = A.H;
     if (gp.lane < 7) {
         const uint2 e1 = touch64(A.ntab + (size_t)g * H + tab_home(h, H));
@@ -874,7 +753,6 @@ __device__ __forceinline__ void warm_expand(const Arena &A, const Grp &gp, int g
         if (nf > 0) { touch32(A.nfree + (size_t)g * M + nf - 1); if (nf > 7) touch32(A.nfree + (size_t)g * M + nf - 7); }
         if (nof > 0) { touch32(A.ofree + (size_t)g * M + nof - 1); if (nof > 7) touch32(A.ofree + (size_t)g * M + nof - 7); }
     }
-#endif
 }
 
 constexpr int STAGE_WORDS = 36;                      // rec[20] | key[12] | h, hk, end, score

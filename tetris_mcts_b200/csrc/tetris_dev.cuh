@@ -165,13 +165,9 @@ __device__ __forceinline__ void lock_piece(Game &g) {   // SPEC §3.3
 // serially by the warp.  The step is therefore written with ONE collision test for all shifting / rotating / soft-drop actions
 // (a candidate position per action, accepted if it does not collide; action 0 proposes the current position) and ONE lock_piece
 // site shared by the hard drop and by gravity; only the hard drop's distance computation is a branch of its own.
-#ifndef B200_PLAY_UNIFIED
-#define B200_PLAY_UNIFIED 1
-#endif
 __device__ __forceinline__ void play(Game &g, int action) {
     if (g.end) return;
     uint32_t shape = shape_of(g.piece, g.rot);
-#if B200_PLAY_UNIFIED
     bool lock = false;
     if (action == 5) {   // hard drop
         const int d = drop_distance(g.w, shape, g.px, g.py);
@@ -197,31 +193,6 @@ __device__ __forceinline__ void play(Game &g, int action) {
         }
     }
     if (lock) lock_piece(g);
-#else
-    if (action == 5) {   // hard drop
-        const int d = drop_distance(g.w, shape, g.px, g.py);
-        g.py += d;
-        if (g.scoring == 0) g.score += 2 * d;
-        g.dropcnt = 0;
-        lock_piece(g);
-        return;
-    }
-    if (action == 1) { if (!collides(g.w, shape, g.px - 1, g.py)) g.px -= 1; }
-    else if (action == 2) { if (!collides(g.w, shape, g.px + 1, g.py)) g.px += 1; }
-    else if (action == 3 || action == 4) {
-        int nr = (g.rot + (action == 3 ? 1 : 3)) & 3;
-        uint32_t ns = shape_of(g.piece, nr);
-        if (!collides(g.w, ns, g.px, g.py)) { g.rot = nr; shape = ns; }
-    } else if (action == 6) {
-        if (!collides(g.w, shape, g.px, g.py + 1)) { g.py += 1; if (g.scoring == 0) g.score += 1; }
-    }
-    g.dropcnt += 1;
-    if (g.dropcnt >= g.app) {
-        g.dropcnt = 0;
-        if (!collides(g.w, shape, g.px, g.py + 1)) g.py += 1;
-        else lock_piece(g);
-    }
-#endif
 }
 
 // ---- SPEC §6 packed record <-> registers

@@ -32,21 +32,7 @@ __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)_
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
-#ifndef B200_MBAR_SUSPEND_NS
-#define B200_MBAR_SUSPEND_NS 0   // > 0: try_wait with this suspend-time hint (fewer turns of the polling loop; see profiles/exp_variants_r2j.txt)
-#endif
 __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-#if B200_MBAR_SUSPEND_NS > 0
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1, %2;\n"
-        "@P1 bra DONE;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}" ::"r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)B200_MBAR_SUSPEND_NS) : "memory");
-#else
     asm volatile(
         "{\n"
         ".reg .pred P1;\n"
@@ -56,16 +42,12 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
         "bra LAB_WAIT;\n"
         "DONE:\n"
         "}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-#endif
 }
 // whole warp waits, one lane polls (32 lanes polling the same word is shared-memory traffic the MMA operand fetch competes with)
 __device__ __forceinline__ void mbar_wait_warp(uint64_t *bar, uint32_t parity);
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-#ifndef B200_MBAR_FASTPATH
-#define B200_MBAR_FASTPATH 1   // most waits of the conv pipeline find their phase already complete: one warp-wide test_wait (a broadcast read)
-#endif                         // answers that without the lane-0 poll + __syncwarp round trip
 __device__ __forceinline__ bool mbar_test(uint64_t *bar, uint32_t parity) {
     uint32_t ok;
     asm volatile(
@@ -77,9 +59,9 @@ __device__ __forceinline__ bool mbar_test(uint64_t *bar, uint32_t parity) {
     return ok != 0u;
 }
 __device__ __forceinline__ void mbar_wait_warp(uint64_t *bar, uint32_t parity) {
-#if B200_MBAR_FASTPATH
+    // most waits of the conv pipeline find their phase already complete: one warp-wide test_wait (a broadcast read) answers that
+    // without the lane-0 poll + __syncwarp round trip
     if (__all_sync(0xffffffffu, mbar_test(bar, parity))) return;
-#endif
     if ((threadIdx.x & 31) == 0) mbar_wait(bar, parity);
     __syncwarp();
 }
@@ -90,14 +72,6 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t by
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
                  "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
-// the same with an L2 eviction policy (search_dev.cuh: l2_policy_stream): act3 is written once and read once
-__device__ __forceinline__ void bulk_g2s_hint(void *dst, const void *src, uint32_t bytes, uint64_t *bar, uint64_t pol) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(pol) : "memory");
-}
-#ifndef B200_L2_STREAM_ACT3
-#define B200_L2_STREAM_ACT3 0   // measured on B200: k_tc_fc -5 %, but the tree kernels that follow +13 % (net loss); kept as a switch
-#endif
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
@@ -194,18 +168,6 @@ __device__ __forceinline__ void split8(const float (&x)[8], uint4 &c1, uint4 &c2
 // conv1 (K = 9 taps, exact {-1,0,1} inputs) runs on the tensor core too from an im2col operand the workers build.
 // (Two independent worker sets of 8 warps x 16 channels on alternating boards, one MMA issuer each, were measured on B200 at 3 204 clk per
 // board against 2 751 with one set — profiles/exp_variants_r2f.txt — and removed.)
-#ifndef B200_CONV3_PAIR
-#define B200_CONV3_PAIR 0                   // 1: conv3 on a transposed grid that holds TWO boards per M = 128 tile (9 MMAs per board instead of 18), see below.
-                                            // Built, parity-green and measured on B200 (profiles/exp_variants_r2i.txt): tensor-pipe cycles -24 %, instructions -8 %, but the
-                                            // kernel is 7-8 % SLOWER (2 750 -> 3 080 clk per board): E3 now runs every other iteration and the 18-MMA burst of a pair
-                                            // lands in front of conv2, so the workers wait longer for c2 than conv3 saves.  Off.
-#endif
-#ifndef B200_CONV3_E3FIRST
-#define B200_CONV3_E3FIRST 0                // worker order inside an iteration: E3 | E2 | E1 instead of E2 | E3 | E1
-#endif
-#ifndef B200_CONV3_XPOSE
-#define B200_CONV3_XPOSE 1                  // the conv2 epilogue re-deals its values across the warp before the store (see there); 0: padded row groups instead
-#endif
 constexpr int TCC_WORKERS = 512;            // warps 0-15: the three epilogues
 constexpr int TCC_ISSUER = TCC_WORKERS / 32; // warp 16: MMA issuer of conv1 + conv2 (one elected lane)
 constexpr int TCC_ISSUER3 = TCC_ISSUER + 1; // warp 17: MMA issuer of conv3.  A 56-clk MMA costs its issuing thread ~8 dependent instructions
@@ -223,39 +185,17 @@ constexpr int TCC_RUN = 4;                  // consecutive requests handed to a 
 constexpr int TCC_ASLOT = 2 * 4 * TCC_R * 16;    // operand buffer of one board: act1 [split][chunk 4][144 rows][16 B]
 constexpr int TCC_IMROWS = 256;             // im2col rows per board: 144 used, two M=128 tiles
 constexpr int TCC_IMSLOT = 2 * TCC_IMROWS * 16;  // [chunk 2][256 rows][16 B] fp16
-#if B200_CONV3_PAIR
-// conv3's output is 14 x 4 pixels: on the 8-wide grid an M = 128 tile carries 56 useful rows.  TRANSPOSED (row = x, 16 columns = y) the output of
-// one board is 4 x 16 = 64 rows, so two boards share a tile:  m = x*32 + (board & 1)*16 + y.  The conv2 epilogue writes act2 in that order
-// (6 x 32 = 192 rows per pair), the A operand of filter column dx is the pair's array started dx*32 rows later, the three VERTICAL taps are
-// stacked along N and summed by the epilogue (y + dy stays inside the board's 16 lanes).  18 MMAs per PAIR of boards.
-// The 8-row groups of the pair array are 144 B apart (SBO; 128 B + 16 B of padding): the conv2 epilogue's 16-byte stores of one pixel row
-// (x = 0..5: 4 groups apart) would otherwise all hit the same banks; with the padding it is a 3-way conflict.
-constexpr int TCC_ACT1_BUFS = 2;            // act1 is no longer overwritten by act2: E1(i) follows E2(i-2) (which waited for conv2(i-2)) in program order
-constexpr int TCC_TSLOTS = 3;               // TMEM: 3 x 128 columns for conv1 / conv2 in turn (conv1(i) is issued after a1(i-1), i.e. after E2(i-3)) + 96 for the pair
-#ifndef B200_CONV3_PSBO
-#define B200_CONV3_PSBO (B200_CONV3_XPOSE ? 128 : 144)
-#endif
-constexpr int TCC_PSBO = B200_CONV3_PSBO;
-constexpr int TCC_PCHUNK = 24 * TCC_PSBO;   // one 8-channel chunk of a pair: 192 rows
-constexpr int TCC_PSLOT = 2 * 4 * TCC_PCHUNK;    // [split][chunk 4][24 row groups][144 B]
-constexpr int TCC_PAIR_BUFS = 2;
-constexpr int TCC_TMEM_PAIR = TCC_TSLOTS * 128;  // first column of the pair accumulator
-#else
-constexpr int TCC_ACT1_BUFS = TCC_SLOTS;    // act2 overwrites the slot's act1 in place (conv2 has finished reading by then)
-constexpr int TCC_TSLOTS = TCC_SLOTS;       // a slot's three accumulators reuse the same 128 columns in turn
-constexpr int TCC_PSLOT = 0;
-constexpr int TCC_PAIR_BUFS = 0;
-#endif
+// act2 overwrites the slot's act1 in place (conv2 has finished reading by then), and a slot's three accumulators reuse the same 128 TMEM
+// columns in turn: board i of a CTA lives in slot i % TCC_SLOTS throughout.
 constexpr int TCC_OFF_W2 = 0;
 constexpr int TCC_OFF_W3 = TCC_OFF_W2 + TCC_WBYTES;
 constexpr int TCC_OFF_W1 = TCC_OFF_W3 + TCC_WBYTES;
 constexpr int TCC_OFF_A1 = TCC_OFF_W1 + TCC_W1BYTES;
-constexpr int TCC_OFF_PAIR = TCC_OFF_A1 + TCC_ACT1_BUFS * TCC_ASLOT;
-constexpr int TCC_OFF_IM = TCC_OFF_PAIR + TCC_PAIR_BUFS * TCC_PSLOT;
+constexpr int TCC_OFF_IM = TCC_OFF_A1 + TCC_SLOTS * TCC_ASLOT;
 constexpr int TCC_OFF_BIAS = TCC_OFF_IM + TCC_SLOTS * TCC_IMSLOT;   // 96 floats
 constexpr int TCC_OFF_KEY = TCC_OFF_BIAS + 96 * 4;                  // TCC_SLOTS x 32 words: the front-end warp's row table (20 rows: settled | piece << 16)
-constexpr int TCC_OFF_BAR = TCC_OFF_KEY + TCC_SLOTS * 32 * 4;       // 7 x TCC_SLOTS mbarriers + tmem pointer
-constexpr int TCC_SMEM = TCC_OFF_BAR + 7 * TCC_SLOTS * 8 + 16;
+constexpr int TCC_OFF_BAR = TCC_OFF_KEY + TCC_SLOTS * 32 * 4;       // 6 x TCC_SLOTS mbarriers + tmem pointer
+constexpr int TCC_SMEM = TCC_OFF_BAR + 6 * TCC_SLOTS * 8 + 16;
 constexpr int TCC_TMEM_COLS = 512;
 constexpr int ACT3_KCHUNKS = 224;           // 1792 / 8
 static_assert(TCC_SMEM <= 227 * 1024, "k_tc_conv shared memory");
@@ -331,27 +271,9 @@ __device__ __forceinline__ void issue_conv_layer(uint32_t tmem_d, uint32_t a_add
     }
 }
 
-#if B200_CONV3_PAIR
-// conv3 of a PAIR of boards (see TCC_PSBO above): for each (dx, channel half): a1*W1, a1*W2, a2*W1; weights n = dy*32 + cout.
-__device__ __forceinline__ void issue_conv3_pair(uint32_t tmem_d, uint32_t a_addr, uint32_t w_addr) {
-    const uint64_t a0 = umma_desc(a_addr, TCC_PCHUNK, TCC_PSBO), b0 = umma_desc(w_addr, 96 * 16, 128);
-    constexpr uint32_t idesc = umma_idesc_f16(128, 96);
-#pragma unroll
-    for (int dx = 0; dx < 3; ++dx) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            const uint32_t a_hi = (2 * h * TCC_PCHUNK + dx * 4 * TCC_PSBO) / 16, a_lo = a_hi + 4 * TCC_PCHUNK / 16;   // 16-byte units
-            const uint32_t b_hi = (dx * 2 + h) * (TCC_WBLOCK / 16), b_lo = b_hi + 2 * 96;
-            umma_f16(tmem_d, a0 + a_hi, b0 + b_hi, idesc, (dx | h) ? 1u : 0u);
-            umma_f16(tmem_d, a0 + a_hi, b0 + b_lo, idesc, 1u);
-            umma_f16(tmem_d, a0 + a_lo, b0 + b_hi, idesc, 1u);
-        }
-    }
-}
-#endif
 
 __global__ void __launch_bounds__(TCC_THREADS, 1)
-k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr, const int32_t *first_ptr, const uint32_t *keys, int M, uint8_t *act3,
+k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr, const uint32_t *keys, int M, uint8_t *act3,
           int n_tiles, unsigned long long *prof) {
 #define PROF_T(i) do { if (prof && do_prof) { long long _n = clock64(); pacc[i] += _n - ptick; ptick = _n; } } while (0)
     extern __shared__ __align__(128) uint8_t smem[];
@@ -360,11 +282,8 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
     constexpr int NS = TCC_SLOTS;
     uint64_t *bar_c1 = bars, *bar_c2 = bars + NS, *bar_c3 = bars + 2 * NS;             // tensor core -> workers: layer of slot done
     uint64_t *bar_a0 = bars + 3 * NS, *bar_a1 = bars + 4 * NS, *bar_a2 = bars + 5 * NS; // workers -> issuer: operand of slot written
-#if B200_CONV3_PAIR
-    uint64_t *bar_e3 = bars + 6 * NS;                                                   // workers -> conv3 issuer: the pair accumulator has been read
-#endif
     uint32_t *sKey = reinterpret_cast<uint32_t *>(smem + TCC_OFF_KEY);
-    uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(smem + TCC_OFF_BAR + 7 * NS * 8);
+    uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(smem + TCC_OFF_BAR + 6 * NS * 8);
     const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
     // ---- one-time setup: weights into smem, zeroed operands, barriers, TMEM
     for (int i = t; i < TCC_WBYTES / 16; i += TCC_THREADS) {
@@ -378,7 +297,6 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
         for (int i = 0; i < 3 * NS; ++i) mbar_init(&bars[i], 1);
         for (int i = 3 * NS; i < 4 * NS; ++i) mbar_init(&bars[i], 1);                      // a0: the front-end warp alone builds the conv1 operand
         for (int i = 4 * NS; i < 6 * NS; ++i) mbar_init(&bars[i], TCC_WORKERS / 32);   // a1, a2: one arrival per worker warp
-        for (int i = 6 * NS; i < 7 * NS; ++i) mbar_init(&bars[i], TCC_WORKERS / 32);          // e3 (entry 0 used): one arrival per worker warp
         fence_barrier_init();
     }
     if (warp == TCC_ISSUER) tmem_alloc<TCC_TMEM_COLS>(tmem_ptr);
@@ -387,8 +305,7 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
-    const int first = first_ptr ? *first_ptr : 0;      // this launch evaluates the requests [first, *n_req_ptr) (the deep lane's: see k_merge_requests)
-    const int n_req = *n_req_ptr - first;
+    const int n_req = *n_req_ptr;
     // Boards are handed out in runs of TCC_RUN consecutive requests (neighbouring act3 rows get written close in time; short runs keep
     // the CTAs' board counts within TCC_RUN of each other: with runs of 8 the last CTAs had 4 % more work); board i of
     // this CTA's sequence lives in slot i % 4.  Four boards are in flight at different stages (software pipeline):
@@ -400,7 +317,7 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
     const int n_runs = (n_req + TCC_RUN - 1) / TCC_RUN;
     int n_local = 0;
     for (int run = blockIdx.x; run < n_runs; run += gridDim.x) n_local += min(TCC_RUN, n_req - run * TCC_RUN);
-    auto board_of = [&](int i) -> int { return first + ((i / TCC_RUN) * (int)gridDim.x + (int)blockIdx.x) * TCC_RUN + (i % TCC_RUN); };
+    auto board_of = [&](int i) -> int { return ((i / TCC_RUN) * (int)gridDim.x + (int)blockIdx.x) * TCC_RUN + (i % TCC_RUN); };
     if (warp == TCC_ISSUER) {
         // ===================================================== MMA issuer
         if (lane == 0) {
@@ -424,15 +341,15 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
                     PROF_T(8);
                     tc_fence_after();
                     const uint64_t a0 = umma_desc(s_im + slot * TCC_IMSLOT, TCC_IMROWS * 16, 128), b0 = umma_desc(s_w1, 64 * 16, 128);
-                    umma_f16(tmem_base + (i % TCC_TSLOTS) * 128, a0, b0, umma_idesc_f16(128, 64), 0u);
-                    umma_f16(tmem_base + (i % TCC_TSLOTS) * 128 + 64, a0 + 128, b0, umma_idesc_f16(128, 64), 0u);
+                    umma_f16(tmem_base + slot * 128, a0, b0, umma_idesc_f16(128, 64), 0u);
+                    umma_f16(tmem_base + slot * 128 + 64, a0 + 128, b0, umma_idesc_f16(128, 64), 0u);
                     umma_commit(&bar_c1[slot]);
                     PROF_T(9);
                 }
                 if (i >= 1) {                                    // conv2 (model_vv.py:34): act1 on the 18x8 grid
                     const int j = i - 1, slot = j % NS;
                     tc_fence_after();
-                    issue_conv_layer(tmem_base + (j % TCC_TSLOTS) * 128, s_act + (j % TCC_ACT1_BUFS) * TCC_ASLOT, s_w2);
+                    issue_conv_layer(tmem_base + slot * 128, s_act + slot * TCC_ASLOT, s_w2);
                     umma_commit(&bar_c2[slot]);
                     PROF_T(11);
                 }
@@ -445,23 +362,6 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
             const uint32_t s_w3 = smem_u32(smem + TCC_OFF_W3);
             const bool do_prof = blockIdx.x == 0;
             long long pacc[16] = {0}, ptick = clock64();
-#if B200_CONV3_PAIR
-            // pair k = boards 2k, 2k+1 of this CTA.  a2 of the pair's LAST board implies (program order of every worker warp) that the other
-            // board's act2 is written and that E3(k-2) (which waited for conv3(k-2)) is done with the pair buffer.  The ONE pair accumulator
-            // is handed back explicitly (e3): a last pair of one board is ready (a2(2k), first phase of iteration 2k+2) before E3(k-1) of
-            // that same iteration has read it.
-            const uint32_t s_pair = smem_u32(smem + TCC_OFF_PAIR);
-            for (int k = 0; 2 * k < n_local; ++k) {
-                const int jl = min(2 * k + 1, n_local - 1);
-                mbar_wait(&bar_a2[jl % NS], (uint32_t)(jl / NS) & 1u);
-                if (k >= 1) mbar_wait(&bar_e3[0], (uint32_t)(k - 1) & 1u);
-                PROF_T(12);
-                tc_fence_after();
-                issue_conv3_pair(tmem_base + TCC_TMEM_PAIR, s_pair + (k % TCC_PAIR_BUFS) * TCC_PSLOT, s_w3);
-                umma_commit(&bar_c3[k & 1]);
-                PROF_T(13);
-            }
-#else
             const uint32_t s_act = smem_u32(smem + TCC_OFF_A1);
             for (int j = 0; j < n_local; ++j) {                  // act2 on the 16x8 grid
                 const int slot = j % NS;
@@ -472,7 +372,6 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
                 umma_commit(&bar_c3[slot]);
                 PROF_T(13);
             }
-#endif
             if (prof && do_prof) for (int i = 12; i < 14; ++i) atomicAdd(&prof[i], (unsigned long long)pacc[i]);
         }
     } else if (warp == TCC_LOADER) {
@@ -545,11 +444,7 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
 #pragma unroll
         for (int e = 0; e < 8; ++e) { bias1[e] = sB[cq * 8 + e] * TC_SCALE_A; bias2[e] = sB[32 + cq * 8 + e] * TC_SCALE_A; bias3[e] = sB[64 + cq * 8 + e] * TC_SCALE_A; }
         constexpr float K23 = TC_UNSCALE * TC_SCALE_A, K1 = TC_SCALE_A / TC_SCALE_W;
-#if B200_CONV3_PAIR
-        const int n_iter = 2 * ((n_local + 1) / 2) + 3;                   // the last pair's E3 runs at iteration 2k+4
-#else
         const int n_iter = n_local + 3;
-#endif
         auto phase_e2 = [&](int i) {
             // ---- E2(i-2): conv2 epilogue: dx sum + bias + ReLU + split -> act2
             if (i >= 2 && i - 2 < n_local) {
@@ -558,39 +453,18 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
                 PROF_T(3);
                 tc_fence_after();
                 float v[8];
-                tmem_ld_conv_sum(t_lane + (j % TCC_TSLOTS) * 128, v);
+                tmem_ld_conv_sum(t_lane + slot * 128, v);
                 {
                     float o[8];
 #pragma unroll
                     for (int e = 0; e < 8; ++e) o[e] = fmaxf(fmaf(v[e], K23, bias2[e]), 0.f);
                     uint4 c1, c2;
                     split8(o, c1, c2);
-#if !B200_CONV3_PAIR
                     if ((m & 7) < 6) {                           // 16x8 grid, in place of the slot's act1
                         uint8_t *base = smem + TCC_OFF_A1 + slot * TCC_ASLOT + (cq * TCC_R + m) * 16;
                         *reinterpret_cast<uint4 *>(base) = c1;
                         *reinterpret_cast<uint4 *>(base + 4 * TCC_R * 16) = c2;
                     }
-#else
-#if B200_CONV3_XPOSE
-                    // The 8 lanes of a store phase hold ONE y and x = 0..7: on the pair grid their rows are 4 groups (512 B) apart, an 8-way bank
-                    // conflict.  Re-deal the warp's 4 y x 8 x values x-major first (lane' = x*4 + yy takes lane yy*8 + x): a phase then holds
-                    // two x and four y (four different 16-byte bank groups), a 2-way conflict, and the row groups stay 128-byte aligned.
-                    const int src = (lane & 3) * 8 + (lane >> 2), xs = lane >> 2, ys = (q << 2) + (lane & 3);
-                    c1.x = __shfl_sync(0xffffffffu, c1.x, src); c1.y = __shfl_sync(0xffffffffu, c1.y, src);
-                    c1.z = __shfl_sync(0xffffffffu, c1.z, src); c1.w = __shfl_sync(0xffffffffu, c1.w, src);
-                    c2.x = __shfl_sync(0xffffffffu, c2.x, src); c2.y = __shfl_sync(0xffffffffu, c2.y, src);
-                    c2.z = __shfl_sync(0xffffffffu, c2.z, src); c2.w = __shfl_sync(0xffffffffu, c2.w, src);
-#else
-                    const int xs = m & 7, ys = m >> 3;           // padded row groups (TCC_PSBO = 144): a 3-way conflict, but the MMA's 128-byte rows straddle lines
-#endif
-                    if (xs < 6) {
-                        const int prow = xs * 32 + (j & 1) * 16 + ys;   // transposed pair grid: x*32 + board*16 + y
-                        uint8_t *base = smem + TCC_OFF_PAIR + ((j >> 1) % TCC_PAIR_BUFS) * TCC_PSLOT + cq * TCC_PCHUNK + (prow >> 3) * TCC_PSBO + (prow & 7) * 16;
-                        *reinterpret_cast<uint4 *>(base) = c1;
-                        *reinterpret_cast<uint4 *>(base + 4 * TCC_PCHUNK) = c2;
-                    }
-#endif
                 }
                 tc_fence_before();
                 fence_async_smem();
@@ -601,18 +475,6 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
         };
         auto phase_e3 = [&](int i) {
             // ---- E3: conv3 epilogue: tap sum + bias + ReLU + split -> act3 in HBM (FC tile layout)
-#if B200_CONV3_PAIR
-            if (i >= 4 && !(i & 1) && i - 4 < n_local) {         // pair k = boards 2k, 2k+1, one iteration after E2(2k+1)
-                const int k = (i - 4) >> 1, j = 2 * k + (lane >> 4);
-                mbar_wait_warp(&bar_c3[k & 1], (uint32_t)(k >> 1) & 1u);
-                PROF_T(5);
-                tc_fence_after();
-                const int y = lane & 15, x = q;                  // TMEM lane m = x*32 + board*16 + y
-                float v[8];
-                tmem_ld_conv_sum(t_lane + TCC_TMEM_PAIR, v);     // the taps stacked along N are the vertical ones here: y + dy = lane + dy
-                if (y < 14 && j < n_local) {
-                    const int ridx = board_of(j);
-#else
             if (i >= 3) {
                 const int j = i - 3, slot = j % NS, ridx = board_of(j);
                 mbar_wait_warp(&bar_c3[slot], (uint32_t)(j / NS) & 1u);
@@ -622,27 +484,16 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
                 float v[8];
                 tmem_ld_conv_sum(t_lane + slot * 128, v);
                 if (y < 14 && x < 4) {
-#endif
                     float o[8];
 #pragma unroll
                     for (int e = 0; e < 8; ++e) o[e] = fmaxf(fmaf(v[e], K23, bias3[e]), 0.f);
                     uint4 c1, c2;
                     split8(o, c1, c2);
                     const int kc = (y * 4 + x) * 4 + cq;
-#if B200_L2_STREAM_ACT3
-                    const uint64_t pol = l2_policy_stream();
-                    stg_hint(reinterpret_cast<int4 *>(act3 + act3_off(0, n_tiles, ridx, kc)), make_int4((int)c1.x, (int)c1.y, (int)c1.z, (int)c1.w), pol);
-                    stg_hint(reinterpret_cast<int4 *>(act3 + act3_off(1, n_tiles, ridx, kc)), make_int4((int)c2.x, (int)c2.y, (int)c2.z, (int)c2.w), pol);
-#else
                     *reinterpret_cast<uint4 *>(act3 + act3_off(0, n_tiles, ridx, kc)) = c1;
                     *reinterpret_cast<uint4 *>(act3 + act3_off(1, n_tiles, ridx, kc)) = c2;
-#endif
                 }
                 tc_fence_before();
-#if B200_CONV3_PAIR
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&bar_e3[0]);
-#endif
                 PROF_T(6);
             }
         };
@@ -653,8 +504,8 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
                 mbar_wait_warp(&bar_c1[slot], (uint32_t)(j / NS) & 1u);
                 PROF_T(1);
                 tc_fence_after();
-                uint8_t *abase = smem + TCC_OFF_A1 + (j % TCC_ACT1_BUFS) * TCC_ASLOT + cq * TCC_R * 16;
-                const uint32_t t_c1 = t_lane + (j % TCC_TSLOTS) * 128;
+                uint8_t *abase = smem + TCC_OFF_A1 + slot * TCC_ASLOT + cq * TCC_R * 16;
+                const uint32_t t_c1 = t_lane + slot * 128;
                 {
                     float w1[8], w2[8], o[8];
                     tmem_ld8x2(t_c1, w1, w2);
@@ -685,11 +536,7 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
             }
         };
         for (int i = 0; i < n_iter; ++i) {
-#if B200_CONV3_PAIR && B200_CONV3_E3FIRST
-            phase_e3(i); phase_e2(i); phase_e1(i);
-#else
             phase_e2(i); phase_e3(i); phase_e1(i);
-#endif
         }
         if (prof && do_prof) for (int i = 0; i < 16; ++i) if (i < 8 || i > 13) atomicAdd(&prof[i], (unsigned long long)pacc[i]);
     }
@@ -747,11 +594,7 @@ k_tc_fc(NetWeights W, TcWeights TW, const uint8_t *act3, int n_tiles_alloc, cons
                     uint8_t *dst = smem + stage * TCF_STAGE;
 #pragma unroll
                     for (int s = 0; s < 2; ++s) {
-#if B200_L2_STREAM_ACT3
-                        bulk_g2s_hint(dst + s * TCF_A_BYTES, act3 + (((size_t)s * n_tiles_alloc + tile) * ACT3_KCHUNKS + 2 * j) * 2048, TCF_A_BYTES, &full[stage], l2_policy_stream());
-#else
                         bulk_g2s(dst + s * TCF_A_BYTES, act3 + (((size_t)s * n_tiles_alloc + tile) * ACT3_KCHUNKS + 2 * j) * 2048, TCF_A_BYTES, &full[stage]);
-#endif
                         bulk_g2s(dst + 2 * TCF_A_BYTES + s * TCF_B_BYTES, TW.wfc + ((size_t)s * TCF_KBLOCKS + j) * TCF_B_BYTES, TCF_B_BYTES, &full[stage]);
                     }
                     if (++stage == TCF_STAGES) { stage = 0; ph ^= 1; }
@@ -852,7 +695,7 @@ static int tc_prepare(void **state, const float *w, cudaStream_t stream) {
                 if (tap < 9) host_split2(c1w[n * 9 + tap] * TC_SCALE_W, s2);
                 for (int s = 0; s < 2; ++s) p1[((size_t)c2 * 64 + s * 32 + n) * 8 + e] = s2[s];
             }
-    for (int layer = 0; layer < 2; ++layer) {                    // conv2/3: [(shift tap, half)][split][chunk][n = stacked tap*32 + cout][8]
+    for (int layer = 0; layer < 2; ++layer) {                    // conv2/3: [(dy, half)][split][chunk][n = dx*32 + cout][8]
         const float *cw = layer ? c3w : c2w;
         uint16_t *dst = layer ? p3 : p2;
         for (int dy = 0; dy < 3; ++dy)
@@ -864,10 +707,8 @@ static int tc_prepare(void **state, const float *w, cudaStream_t stream) {
                                 int ci = 16 * hh + 8 * c2 + e;
                                 uint16_t s2[2];
                                 host_split2(cw[(n * 32 + ci) * 9 + dy * 3 + dx] * TC_SCALE_W, s2);
-                                // the tap that shifts the A operand selects the block, the other one is stacked along N (conv3 in pair mode: transposed)
-                                const int shift_tap = (layer && B200_CONV3_PAIR) ? dx : dy, n_tap = (layer && B200_CONV3_PAIR) ? dy : dx;
-                                for (int s = 0; s < 2; ++s)
-                                    dst[(((((size_t)(shift_tap * 2 + hh)) * 2 + s) * 2 + c2) * 96 + n_tap * 32 + n) * 8 + e] = s2[s];
+                                for (int s = 0; s < 2; ++s)   // dy shifts the A operand and selects the block, dx is stacked along N
+                                    dst[(((((size_t)(dy * 2 + hh)) * 2 + s) * 2 + c2) * 96 + dx * 32 + n) * 8 + e] = s2[s];
                             }
     }
     for (int j = 0; j < TCF_KBLOCKS; ++j)

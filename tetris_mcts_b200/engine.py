@@ -115,10 +115,6 @@ class BatchedEngine:
         L.check(L.lib().b200_set_path_cache(self.h, int(bool(on))))
         self.path_cache = bool(on)
 
-    def set_deep_lane(self, max_games):
-        """Scheduling only: the max_games games with the longest traces walk on a second stream (b200_set_deep_lane); 0 = off."""
-        L.check(L.lib().b200_set_deep_lane(self.h, int(max_games)))
-
     def update_root(self, auto_reset=False):
         L.check(L.lib().b200_update_root(self.h, int(auto_reset)))
 
