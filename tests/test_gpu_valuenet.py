@@ -64,6 +64,23 @@ def test_matches_reference_golden(gpu_lib, oracle, kind):
         eng.close()
 
 
+def test_tensor_core_path_matches_cuda_core_path(gpu_lib, oracle):
+    """Every batch size from one board to two or three 128-board FC tiles per CTA (40000 boards = 313 tiles), position-independent."""
+    from tetris_mcts_b200.engine import BatchedEngine
+    w = oracle.seeded_weights(3)
+    et = BatchedEngine(1, max_nodes=64, eval_kind="net_tc", weights=w)
+    es = BatchedEngine(1, max_nodes=64, eval_kind="net", weights=w)
+    for n in (1, 129, 700, 20000, 40000):
+        s = boards(n, n)
+        (vt, rt), (vs, rs) = et.valuenet(s), es.valuenet(s)
+        assert np.allclose(vt, vs, rtol=RTOL, atol=ATOL), (n, np.abs(vt - vs).max())
+        assert np.allclose(rt, rs, rtol=RTOL, atol=ATOL), (n, np.abs(rt - rs).max())
+        if n == 700:
+            v2, r2 = et.valuenet(s[::-1])
+            assert np.array_equal(v2[::-1], vt) and np.array_equal(r2[::-1], rt)
+    et.close(); es.close()
+
+
 def test_tensor_core_conv_stack_matches_cuda_core_path(gpu_lib, oracle):
     """Layer-level check of the tcgen05 shift-GEMM convolutions: the flatten input of fc1 from both device paths."""
     import ctypes as C

@@ -50,9 +50,10 @@ struct b200_engine {
     bool have_weights = false;
     float *d_wraw = nullptr;
     NetWeights W{};
-    float *d_act3 = nullptr; size_t act3_rows = 0;
-    void *tc_state = nullptr; void *dn_tc_state = nullptr;
+    float *d_act3 = nullptr; size_t act3_rows = 0;                                            // CUDA-core path
+    uint8_t *d_tcw = nullptr; TcWeights TW{}; uint8_t *d_act3_tc = nullptr; size_t act3_tiles = 0;    // tensor-core path
     bool have_dist_weights = false; float *d_dnw = nullptr; DistNetWeights DW{}; float *d_dn_act = nullptr; size_t dn_rows = 0;
+    uint8_t *d_dn_tcw = nullptr; DnTcWeights DTW{}; uint8_t *d_dn_act_tc = nullptr; size_t dn_act_tiles = 0;
     int n_sm = 148;
     // timing
     bool timing = false;
@@ -252,8 +253,6 @@ extern "C" int b200_engine_destroy(b200_engine *e) {
     if (!e) return B200_OK;
     if (e->stream) cudaStreamSynchronize(e->stream);
     if (e->step_exec) cudaGraphExecDestroy(e->step_exec);
-    tc_destroy(e->tc_state);
-    dn_tc_destroy(e->dn_tc_state);
     for (void *p : e->allocs) cudaFree(p);
     for (auto &ev : e->ev) cudaEventDestroy(ev);
     if (e->t0) { cudaEventDestroy(e->t0); cudaEventDestroy(e->t1); }
@@ -325,49 +324,46 @@ extern "C" int b200_load_weights(b200_engine *e, const float *w) {
     e->W.wfc1 = e->W.b1 + 96; e->W.bfc1 = e->W.wfc1 + (size_t)1792 * 256; e->W.wout = e->W.bfc1 + 256;
     e->W.bout = e->W.wout + 512; e->W.ub = e->W.bout + 2; e->W.lb = e->W.bout + 4;
     CK(cudaFuncSetAttribute(k_vn_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, VN_SMEM_BYTES));
-    {
-        int rc = tc_prepare(&e->tc_state, w, e->stream);
-        if (rc) return fail(B200_ERR_CUDA, "tensor-core weight preparation failed");
-    }
+    if (!e->d_tcw && dalloc(e, &e->d_tcw, TC_PACKED_BYTES, false)) return B200_ERR_CUDA;
+    if (tc_prepare(w, e->d_tcw, e->TW, e->stream)) return fail(B200_ERR_CUDA, "tensor-core weight preparation failed");
     e->have_weights = true;
     drop_step_graph(e);
     return B200_OK;
 }
 
-static int ensure_act3(b200_engine *e, size_t rows) {
-    if (e->act3_rows >= rows) return 0;
-    if (e->d_act3) { cudaStreamSynchronize(e->stream); dfree(e, e->d_act3); e->d_act3 = nullptr; e->act3_rows = 0; }
-    if (dalloc(e, &e->d_act3, rows * 1792, false)) return B200_ERR_CUDA;
-    e->act3_rows = rows;
+// Grow a network's activation buffer to `need` units of `unit` elements.  A replaced buffer (a larger standalone batch) is only freed once
+// the stream has drained, and the captured step graph, which holds its address, is dropped.
+template <typename T>
+static int grow_act(b200_engine *e, T **buf, size_t *have, size_t need, size_t unit, bool zero) {
+    if (*have >= need) return 0;
+    const bool moved = *buf != nullptr;
+    if (moved) { cudaStreamSynchronize(e->stream); dfree(e, *buf); *buf = nullptr; *have = 0; }
+    if (dalloc(e, buf, need * unit, zero)) return B200_ERR_CUDA;
+    *have = need;
+    if (moved) drop_step_graph(e);
     return 0;
 }
+static inline size_t tiles_of(size_t rows) { return (rows + 127) / 128; }
 
 // run the network over the request list req[0..*n_req) -> eval_out; device-side count, no host sync
 static int launch_net(b200_engine *e, const uint2 *req, const int32_t *n_req, const uint32_t *keys, int M, float2 *eval_out,
                       size_t max_rows) {
     if (!e->have_weights) return fail(B200_ERR_NO_WEIGHTS, "b200_load_weights was not called");
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
-        TcState *st = (TcState *)e->tc_state;
-        const uint8_t *act3_before = st->d_act3;
-        if (tc_ensure_act3(st, max_rows, e->stream)) return fail(B200_ERR_CUDA, "act3 (tensor-core layout) allocation failed");
-        if (act3_before && st->d_act3 != act3_before) drop_step_graph(e);   // a larger standalone batch moved the activation buffer
+        if (grow_act(e, &e->d_act3_tc, &e->act3_tiles, tiles_of(max_rows), TcfPipe::ACT_TILE_BYTES, true)) return B200_ERR_CUDA;
         {
             PhaseTimer t(e, PH_CONV);
-            k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, e->stream>>>(e->W, st->TW, req, n_req, keys, M, st->d_act3, (int)st->tiles,
+            k_tc_conv<<<e->n_sm, TCC_THREADS, TCC_SMEM, e->stream>>>(e->W, e->TW, req, n_req, keys, M, e->d_act3_tc, (int)e->act3_tiles,
                                                                     e->timing ? e->A.counters + 16 : nullptr);
         }
         {
             PhaseTimer t(e, PH_FC);
-            k_tc_fc<<<e->n_sm, TCF_THREADS, TCF_SMEM, e->stream>>>(e->W, st->TW, st->d_act3, (int)st->tiles, req, n_req, eval_out);
+            k_tc_fc<<<e->n_sm, FC_PIPE_THREADS, TCF_SMEM, e->stream>>>(e->W, e->TW, e->d_act3_tc, (int)e->act3_tiles, req, n_req, eval_out);
         }
         CK(cudaGetLastError());
         return B200_OK;
     }
-    {
-        const float *act3_before = e->d_act3;
-        if (ensure_act3(e, max_rows)) return B200_ERR_CUDA;
-        if (act3_before && e->d_act3 != act3_before) drop_step_graph(e);
-    }
+    if (grow_act(e, &e->d_act3, &e->act3_rows, max_rows, 1792, false)) return B200_ERR_CUDA;
     {
         PhaseTimer t(e, PH_CONV);
         k_vn_conv<<<e->n_sm, VN_THREADS, VN_SMEM_BYTES, e->stream>>>(e->W, req, n_req, keys, M, e->d_act3);
@@ -383,6 +379,16 @@ static int launch_net(b200_engine *e, const uint2 *req, const int32_t *n_req, co
 // ---------------------------------------------------------------------------------------------------- distributional network
 __global__ void k_states_to_keys(const int8_t *states, int k, uint32_t *keys, uint2 *req);   // defined with the standalone value net below
 
+// standalone forward: k boards -> device keys and one request per board (buffers of `rows` >= k entries), request count k on the device
+static int stage_boards(b200_engine *e, Scratch &tmp, const int8_t *states, int k, size_t rows, uint32_t **d_keys, uint2 **d_req, int32_t **d_n) {
+    int8_t *d_states = nullptr;
+    CK(tmp.get(&d_states, (size_t)k * 200)); CK(tmp.get(d_keys, rows * KEY_WORDS * 4)); CK(tmp.get(d_req, rows * 8)); CK(tmp.get(d_n, 4));
+    CK(cudaMemcpyAsync(d_states, states, (size_t)k * 200, cudaMemcpyHostToDevice, e->stream));
+    CK(cudaMemcpyAsync(*d_n, &k, 4, cudaMemcpyHostToDevice, e->stream));
+    k_states_to_keys<<<(k + 127) / 128, 128, 0, e->stream>>>(d_states, k, *d_keys, *d_req);
+    return B200_OK;
+}
+
 extern "C" int b200_load_dist_weights(b200_engine *e, const float *w, int atoms) {
     if (!e || !w || atoms < 2 || atoms > 64) return fail(B200_ERR_BAD_ARG, "bad argument");
     CK(cudaSetDevice(e->cfg.device));
@@ -395,7 +401,8 @@ extern "C" int b200_load_dist_weights(b200_engine *e, const float *w, int atoms)
     e->DW = dn_pointers(e->d_dnw, atoms);
     CK(cudaFuncSetAttribute(k_dn_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, DN_CONV_SMEM));
     CK(cudaFuncSetAttribute(k_dn_fc, cudaFuncAttributeMaxDynamicSharedMemorySize, DN_FC_SMEM));
-    if (dn_tc_prepare(&e->dn_tc_state, w, atoms, e->stream)) return fail(B200_ERR_CUDA, "tensor-core weight preparation (distributional network) failed");
+    if (!e->d_dn_tcw && dalloc(e, &e->d_dn_tcw, DN_TC_PACKED_BYTES, false)) return B200_ERR_CUDA;
+    if (dn_tc_prepare(w, e->d_dn_tcw, e->DTW, e->stream)) return fail(B200_ERR_CUDA, "tensor-core weight preparation (distributional network) failed");
     e->have_dist_weights = true;
     drop_step_graph(e);
     return B200_OK;
@@ -404,28 +411,19 @@ extern "C" int b200_load_dist_weights(b200_engine *e, const float *w, int atoms)
 static int launch_distnet_on(b200_engine *e, const uint2 *req, const int32_t *n_req, const uint32_t *keys, int M, float *out, size_t max_rows) {
     if (!e->have_dist_weights) return fail(B200_ERR_NO_WEIGHTS, "b200_load_dist_weights was not called");
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
-        DnTcState *st = (DnTcState *)e->dn_tc_state;
-        bool moved = false;
-        if (dn_tc_ensure_act2(st, max_rows, e->stream, &moved)) return fail(B200_ERR_CUDA, "act2 (tensor-core layout) allocation failed");
-        if (moved) drop_step_graph(e);
+        if (grow_act(e, &e->d_dn_act_tc, &e->dn_act_tiles, tiles_of(max_rows), TdfPipe::ACT_TILE_BYTES, true)) return B200_ERR_CUDA;
         {
             PhaseTimer t(e, PH_CONV);
-            k_tdc_conv<<<e->n_sm, TDC_THREADS, TDC_SMEM, e->stream>>>(e->DW, st->TW, req, n_req, keys, M, st->d_act2, (int)st->tiles);
+            k_tdc_conv<<<e->n_sm, TDC_THREADS, TDC_SMEM, e->stream>>>(e->DW, e->DTW, req, n_req, keys, M, e->d_dn_act_tc, (int)e->dn_act_tiles);
         }
         {
             PhaseTimer t(e, PH_FC);
-            k_tdc_fc<<<e->n_sm, TDF_THREADS, TDF_SMEM, e->stream>>>(e->DW, st->TW, st->d_act2, (int)st->tiles, req, n_req, out);
+            k_tdc_fc<<<e->n_sm, FC_PIPE_THREADS, TDF_SMEM, e->stream>>>(e->DW, e->DTW, e->d_dn_act_tc, (int)e->dn_act_tiles, req, n_req, out);
         }
         CK(cudaGetLastError());
         return B200_OK;
     }
-    if (e->dn_rows < max_rows) {
-        const bool had = e->d_dn_act != nullptr;
-        if (had) { cudaStreamSynchronize(e->stream); dfree(e, e->d_dn_act); e->d_dn_act = nullptr; e->dn_rows = 0; }
-        if (dalloc(e, &e->d_dn_act, max_rows * 2048, false)) return B200_ERR_CUDA;
-        e->dn_rows = max_rows;
-        if (had) drop_step_graph(e);
-    }
+    if (grow_act(e, &e->d_dn_act, &e->dn_rows, max_rows, 2048, false)) return B200_ERR_CUDA;
     {
         PhaseTimer t(e, PH_CONV);
         k_dn_conv<<<e->n_sm * 2, DN_THREADS, DN_CONV_SMEM, e->stream>>>(e->DW, req, n_req, keys, M, e->d_dn_act);
@@ -445,13 +443,10 @@ static int launch_distnet(b200_engine *e) {
 extern "C" int b200_distnet_forward(b200_engine *e, const int8_t *states, int k, int atoms, float *dist) {
     if (!e || !states || !dist || k < 1 || atoms != e->DW.atoms) return fail(B200_ERR_BAD_ARG, "bad argument (atoms must match the loaded weights)");
     CK(cudaSetDevice(e->cfg.device));
-    int8_t *d_states = nullptr; uint32_t *d_keys = nullptr; uint2 *d_req = nullptr; int32_t *d_n = nullptr; float *d_out = nullptr;
+    uint32_t *d_keys = nullptr; uint2 *d_req = nullptr; int32_t *d_n = nullptr; float *d_out = nullptr;
     Scratch tmp;
-    CK(tmp.get(&d_states, (size_t)k * 200)); CK(tmp.get(&d_keys, (size_t)k * KEY_WORDS * 4)); CK(tmp.get(&d_req, (size_t)k * 8));
-    CK(tmp.get(&d_n, 4)); CK(tmp.get(&d_out, (size_t)k * atoms * 4));
-    CK(cudaMemcpyAsync(d_states, states, (size_t)k * 200, cudaMemcpyHostToDevice, e->stream));
-    CK(cudaMemcpyAsync(d_n, &k, 4, cudaMemcpyHostToDevice, e->stream));
-    k_states_to_keys<<<(k + 127) / 128, 128, 0, e->stream>>>(d_states, k, d_keys, d_req);
+    if (int rc = stage_boards(e, tmp, states, k, (size_t)k, &d_keys, &d_req, &d_n)) return rc;
+    CK(tmp.get(&d_out, (size_t)k * atoms * 4));
     k_dn_req_rows<<<(k + 127) / 128, 128, 0, e->stream>>>(d_req, k);      // request i -> output row i
     int rc = launch_distnet_on(e, d_req, d_n, d_keys, 0, d_out, (size_t)k);
     if (rc == B200_OK) {
@@ -851,14 +846,11 @@ extern "C" int b200_valuenet_forward(b200_engine *e, const int8_t *states, int k
     if (!e || !states || !v || !var || k < 1) return fail(B200_ERR_BAD_ARG, "bad argument");
     if (k >= (1 << 28)) return fail(B200_ERR_BAD_ARG, "k too large");
     CK(cudaSetDevice(e->cfg.device));
-    int8_t *d_states = nullptr; uint32_t *d_keys = nullptr; uint2 *d_req = nullptr; int32_t *d_n = nullptr; float2 *d_out = nullptr;
+    uint32_t *d_keys = nullptr; uint2 *d_req = nullptr; int32_t *d_n = nullptr; float2 *d_out = nullptr;
     size_t kp = ((size_t)k + 7) & ~(size_t)7;
     Scratch tmp;
-    CK(tmp.get(&d_states, (size_t)k * 200)); CK(tmp.get(&d_keys, kp * KEY_WORDS * 4)); CK(tmp.get(&d_req, kp * 8));
-    CK(tmp.get(&d_n, 4)); CK(tmp.get(&d_out, kp * 8));
-    CK(cudaMemcpyAsync(d_states, states, (size_t)k * 200, cudaMemcpyHostToDevice, e->stream));
-    CK(cudaMemcpyAsync(d_n, &k, 4, cudaMemcpyHostToDevice, e->stream));
-    k_states_to_keys<<<(k + 127) / 128, 128, 0, e->stream>>>(d_states, k, d_keys, d_req);
+    if (int rc = stage_boards(e, tmp, states, k, kp, &d_keys, &d_req, &d_n)) return rc;
+    CK(tmp.get(&d_out, kp * 8));
     // keys are addressed as keys[(game * M + obs)]: with game = i/8 we pass M = 0 so that only obs (= i) indexes
     int rc = launch_net(e, d_req, d_n, d_keys, 0, d_out, kp);
     if (rc == B200_OK) {
@@ -879,16 +871,14 @@ extern "C" int b200_debug_act3(b200_engine *e, const int8_t *states, int k, floa
     int rc = b200_valuenet_forward(e, states, k, v.data(), var.data());   // leaves act3 of these k boards in the scratch buffers
     if (rc) return rc;
     if (e->cfg.eval_kind == B200_EVAL_NET_TC) {
-        TcState *st = (TcState *)e->tc_state;
-        size_t bytes = (size_t)2 * st->tiles * ACT3_KCHUNKS * 2048;
-        std::vector<uint8_t> h(bytes);
-        CK(cudaMemcpy(h.data(), st->d_act3, bytes, cudaMemcpyDeviceToHost));
+        std::vector<uint8_t> h(e->act3_tiles * TcfPipe::ACT_TILE_BYTES);
+        CK(cudaMemcpy(h.data(), e->d_act3_tc, h.size(), cudaMemcpyDeviceToHost));
         for (int r = 0; r < k; ++r)
             for (int kp = 0; kp < 1792; ++kp) {
                 int p = kp >> 5, c = kp & 31;
                 float sum = 0.f;
                 for (int s = 1; s >= 0; --s) {
-                    size_t off = ((((size_t)s * st->tiles + (r >> 7)) * ACT3_KCHUNKS + (kp >> 3)) * 128 + (r & 127)) * 16 + (kp & 7) * 2;
+                    size_t off = ((((size_t)s * e->act3_tiles + (r >> 7)) * ACT3_KCHUNKS + (kp >> 3)) * 128 + (r & 127)) * 16 + (kp & 7) * 2;
                     uint16_t hb; memcpy(&hb, &h[off], 2);
                     sum += host_half_f(hb);
                 }

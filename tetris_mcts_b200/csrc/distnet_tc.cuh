@@ -7,7 +7,7 @@
 //               started dy*8 rows later, the four horizontal taps stacked along N = 128, 4 dy x 2 channel halves x 3 split products = 24
 //               tcgen05.mma (M=128, N=128, K=16); the epilogue sums the taps with three lane shuffles, applies bias + LeakyReLU(0.01),
 //               re-splits and writes act2 (16x4 pixels x 32 channels = 2048 per board) to HBM in k_tdc_fc's tile layout.
-//   k_tdc_fc    [R,2048] x [2048,128] like k_tc_fc (1-D TMA ring, warp-specialised); epilogue: bias + LeakyReLU -> fc_v (128 x atoms, CUDA
+//   k_tdc_fc    [R,2048] x [2048,128] on fc_pipeline (valuenet_tc.cuh) like k_tc_fc; epilogue: bias + LeakyReLU -> fc_v (128 x atoms, CUDA
 //               cores, weights in shared memory) -> softmax (model_distributional.py:47-50) -> dist[game][atoms].
 #pragma once
 #include "valuenet_tc.cuh"
@@ -268,205 +268,73 @@ k_tdc_conv(DistNetWeights W, DnTcWeights TW, const uint2 *req, const int32_t *n_
 }
 
 // ---------------------------------------------------------------------------------------------------- fc1 + fc_v + softmax
-constexpr int TDF_THREADS = 192;            // warp 0 producer, warp 1 MMA issuer, warps 2-5 epilogue
-constexpr int TDF_STAGES = 8;
-constexpr int TDF_A_BYTES = 2 * 128 * 16;   // one split of one k16 block of the A tile
-constexpr int TDF_B_BYTES = 2 * 128 * 16;
-constexpr int TDF_STAGE = 2 * TDF_A_BYTES + 2 * TDF_B_BYTES;   // 16384
-constexpr int TDF_KBLOCKS = 128;            // 2048 / 16
+using TdfPipe = FcPipe<128, DACT2_KCHUNKS / 2, 8>;
 constexpr int TDF_ATOMS = 64;               // fc_v columns carried per thread (atoms <= 64, the rest zero)
-constexpr int TDF_OFF_BAR = TDF_STAGES * TDF_STAGE;
-constexpr int TDF_OFF_EPI = TDF_OFF_BAR + 256;                 // bias[128] | wv[128][64] | bv[64]
-static_assert((2 * TDF_STAGES + 2) * 8 + 4 <= 256, "barrier block overflows into the epilogue constants");
-constexpr int TDF_SMEM = TDF_OFF_EPI + (128 + 128 * TDF_ATOMS + TDF_ATOMS) * 4;
-constexpr int TDF_TMEM_COLS = 128;
+constexpr int TDF_SMEM = TdfPipe::OFF_EPI + (128 + 128 * TDF_ATOMS + TDF_ATOMS) * 4;   // bias[128] | wv[128][64] | bv[64]
 
-__global__ void __launch_bounds__(TDF_THREADS, 1)
+__global__ void __launch_bounds__(FC_PIPE_THREADS, 1)
 k_tdc_fc(DistNetWeights W, DnTcWeights TW, const uint8_t *act2, int n_tiles_alloc, const uint2 *req, const int32_t *n_req_ptr, float *out) {
     extern __shared__ __align__(128) uint8_t smem[];
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem + TDF_OFF_BAR);
-    uint64_t *empty = full + TDF_STAGES;
-    uint64_t *acc_full = empty + TDF_STAGES;
-    uint64_t *acc_empty = acc_full + 1;
-    uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(acc_empty + 1);
-    float *sBias = reinterpret_cast<float *>(smem + TDF_OFF_EPI), *sWv = sBias + 128, *sBv = sWv + 128 * TDF_ATOMS;
-    const int t = threadIdx.x, warp = t >> 5, lane = t & 31, atoms = W.atoms;
-    for (int i = t; i < 128; i += TDF_THREADS) sBias[i] = W.bf1[i];
-    for (int i = t; i < 128 * TDF_ATOMS; i += TDF_THREADS) { const int k = i / TDF_ATOMS, a = i - k * TDF_ATOMS; sWv[i] = a < atoms ? W.wfv[(size_t)k * atoms + a] : 0.f; }
-    if (t < TDF_ATOMS) sBv[t] = t < atoms ? W.bfv[t] : 0.f;
-    if (t == 0) {
-        for (int i = 0; i < TDF_STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        mbar_init(acc_full, 1);
-        mbar_init(acc_empty, 128);
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc<TDF_TMEM_COLS>(tmem_ptr);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr;
-    const int n_req = *n_req_ptr;
-    const int n_tiles = (n_req + 127) >> 7;
-    if (warp == 0) {
-        if (lane == 0) {   // ===== producer: bulk copies of the pre-laid-out operand blocks
-            int stage = 0; uint32_t ph = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                for (int j = 0; j < TDF_KBLOCKS; ++j) {
-                    mbar_wait(&empty[stage], ph ^ 1);
-                    mbar_expect_tx(&full[stage], TDF_STAGE);
-                    uint8_t *dst = smem + stage * TDF_STAGE;
+    float *sBias = reinterpret_cast<float *>(smem + TdfPipe::OFF_EPI), *sWv = sBias + 128, *sBv = sWv + 128 * TDF_ATOMS;
+    const int atoms = W.atoms;
+    auto load_consts = [=](int t) {   // by value: with `atoms` by reference the fc_v index below becomes a 64-bit multiply
+        for (int i = t; i < 128; i += FC_PIPE_THREADS) sBias[i] = W.bf1[i];
+        for (int i = t; i < 128 * TDF_ATOMS; i += FC_PIPE_THREADS) { const int k = i / TDF_ATOMS, a = i - k * TDF_ATOMS; sWv[i] = a < atoms ? W.wfv[(size_t)k * atoms + a] : 0.f; }
+        if (t < TDF_ATOMS) sBv[t] = t < atoms ? W.bfv[t] : 0.f;
+    };
+    fc_pipeline<TdfPipe>(act2, n_tiles_alloc, TW.wfc, n_req_ptr, load_consts, [&](uint32_t taddr, int tile, int row, int n_req, auto drained) {
+        float lg[TDF_ATOMS];
 #pragma unroll
-                    for (int s = 0; s < 2; ++s) {
-                        bulk_g2s(dst + s * TDF_A_BYTES, act2 + (((size_t)s * n_tiles_alloc + tile) * DACT2_KCHUNKS + 2 * j) * 2048, TDF_A_BYTES, &full[stage]);
-                        bulk_g2s(dst + 2 * TDF_A_BYTES + s * TDF_B_BYTES, TW.wfc + ((size_t)s * TDF_KBLOCKS + j) * TDF_B_BYTES, TDF_B_BYTES, &full[stage]);
-                    }
-                    if (++stage == TDF_STAGES) { stage = 0; ph ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {   // ===== MMA issuer: D[128 x 128] += A[128 x 16] * B[128 x 16]^T, three split terms per k block
-            const uint32_t idesc = umma_idesc_f16(128, 128);
-            int stage = 0; uint32_t ph = 0, aph = 0;
-            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                mbar_wait(acc_empty, aph ^ 1);
-                tc_fence_after();
-                uint32_t acc = 0;
-                for (int j = 0; j < TDF_KBLOCKS; ++j) {
-                    mbar_wait(&full[stage], ph);
-                    tc_fence_after();
-                    const uint32_t sbase = smem_u32(smem + stage * TDF_STAGE);
-#pragma unroll
-                    for (int term = 0; term < 3; ++term) {   // a1*b2, a2*b1, a1*b1 (small terms first)
-                        const int sa = term == 1 ? 1 : 0, sb = term == 0 ? 1 : 0;
-                        uint64_t ad = umma_desc(sbase + sa * TDF_A_BYTES, 128 * 16, 128);
-                        uint64_t bd = umma_desc(sbase + 2 * TDF_A_BYTES + sb * TDF_B_BYTES, 128 * 16, 128);
-                        umma_f16(tmem_base, ad, bd, idesc, acc);
-                        acc = 1;
-                    }
-                    umma_commit(&empty[stage]);
-                    if (++stage == TDF_STAGES) { stage = 0; ph ^= 1; }
-                }
-                umma_commit(acc_full);
-                aph ^= 1;
-            }
-        }
-    } else {   // ===== epilogue warps 2..5: TMEM quadrant = warp % 4, one board per thread
-        const int q = warp & 3, row = q * 32 + lane;
-        uint32_t aph = 0;
-        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-            mbar_wait(acc_full, aph);
-            tc_fence_after();
-            float lg[TDF_ATOMS];
-#pragma unroll
-            for (int a = 0; a < TDF_ATOMS; ++a) lg[a] = sBv[a];
+        for (int a = 0; a < TDF_ATOMS; ++a) lg[a] = sBv[a];
 #pragma unroll 1
-            for (int c0 = 0; c0 < 128; c0 += 8) {
-                float v[8];
-                tmem_ld8(tmem_base + ((uint32_t)(q * 32) << 16) + c0, v);
+        for (int c0 = 0; c0 < 128; c0 += 8) {
+            float v[8];
+            tmem_ld8(taddr + c0, v);
 #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float h = leaky(v[j] * TC_UNSCALE + sBias[c0 + j]);          // model_distributional.py:43-44
-                    const float4 *wv = reinterpret_cast<const float4 *>(sWv + (c0 + j) * TDF_ATOMS);
+            for (int j = 0; j < 8; ++j) {
+                const float h = leaky(v[j] * TC_UNSCALE + sBias[c0 + j]);          // model_distributional.py:43-44
+                const float4 *wv = reinterpret_cast<const float4 *>(sWv + (c0 + j) * TDF_ATOMS);
 #pragma unroll
-                    for (int a4 = 0; a4 < TDF_ATOMS / 4; ++a4) {                        // :45 (ascending k, like the CUDA-core kernel)
-                        const float4 w4 = wv[a4];
-                        lg[4 * a4] = fmaf(h, w4.x, lg[4 * a4]); lg[4 * a4 + 1] = fmaf(h, w4.y, lg[4 * a4 + 1]);
-                        lg[4 * a4 + 2] = fmaf(h, w4.z, lg[4 * a4 + 2]); lg[4 * a4 + 3] = fmaf(h, w4.w, lg[4 * a4 + 3]);
-                    }
+                for (int a4 = 0; a4 < TDF_ATOMS / 4; ++a4) {                        // :45 (ascending k, like the CUDA-core kernel)
+                    const float4 w4 = wv[a4];
+                    lg[4 * a4] = fmaf(h, w4.x, lg[4 * a4]); lg[4 * a4 + 1] = fmaf(h, w4.y, lg[4 * a4 + 1]);
+                    lg[4 * a4 + 2] = fmaf(h, w4.z, lg[4 * a4 + 2]); lg[4 * a4 + 3] = fmaf(h, w4.w, lg[4 * a4 + 3]);
                 }
             }
-            tc_fence_before();
-            mbar_arrive(acc_empty);
-            const int ridx = tile * 128 + row;
-            if (ridx < n_req) {                                                        // F.softmax(x, 1), :47-50
-                float mx = -INFINITY;
-#pragma unroll
-                for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) mx = fmaxf(mx, lg[a]);
-                float sum = 0.f;
-#pragma unroll
-                for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) { lg[a] = expf(lg[a] - mx); sum += lg[a]; }
-                float *dst = out + (size_t)req[ridx].x * atoms;
-#pragma unroll
-                for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) dst[a] = lg[a] / sum;
-            }
-            aph ^= 1;
         }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) tmem_dealloc<TDF_TMEM_COLS>(tmem_base);
+        drained();
+        const int ridx = tile * 128 + row;
+        if (ridx < n_req) {                                                        // F.softmax(x, 1), :47-50
+            float mx = -INFINITY;
+#pragma unroll
+            for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) mx = fmaxf(mx, lg[a]);
+            float sum = 0.f;
+#pragma unroll
+            for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) { lg[a] = expf(lg[a] - mx); sum += lg[a]; }
+            float *dst = out + (size_t)req[ridx].x * atoms;
+#pragma unroll
+            for (int a = 0; a < TDF_ATOMS; ++a) if (a < atoms) dst[a] = lg[a] / sum;
+        }
+    });
 }
 
 // ---------------------------------------------------------------------------------------------------- host side
-struct DnTcState {
-    uint8_t *d_w = nullptr;      // wc1 | wc2 | wfc
-    DnTcWeights TW{};
-    uint8_t *d_act2 = nullptr; size_t tiles = 0;
-};
+constexpr size_t DN_TC_PACKED_BYTES = TDC_W1BYTES + (size_t)TDC_WBYTES + (size_t)2 * TdfPipe::KBLOCKS * TdfPipe::B_BYTES;   // wc1 | wc2 | wfc
 
-// w = the state_dict-order weight vector of model_distributional.py (see dn_relayout).  Pure re-layout + fp16 splitting.
-static int dn_tc_prepare(void **state, const float *w, int atoms, cudaStream_t stream) {
-    DnTcState *st = (DnTcState *)*state;
-    if (!st) { st = new DnTcState(); *state = st; }
+// w = the state_dict-order weight vector of model_distributional.py (see dn_relayout), packed into d_w (DN_TC_PACKED_BYTES)
+static int dn_tc_prepare(const float *w, uint8_t *d_w, DnTcWeights &TW, cudaStream_t stream) {
     const float *c1w = w, *c2w = c1w + 512 + 32, *f1w = c2w + 16384 + 32;
-    (void)atoms;
-    const size_t fc_bytes = (size_t)2 * TDF_KBLOCKS * TDF_B_BYTES;
-    std::vector<uint8_t> h(TDC_W1BYTES + (size_t)TDC_WBYTES + fc_bytes);
-    uint16_t *p1 = reinterpret_cast<uint16_t *>(h.data()), *p2 = reinterpret_cast<uint16_t *>(h.data() + TDC_W1BYTES);
-    uint16_t *pf = reinterpret_cast<uint16_t *>(h.data() + TDC_W1BYTES + TDC_WBYTES);
-    for (int c2 = 0; c2 < 2; ++c2)                               // conv1: [chunk][n = split*32 + cout][8], k = tap = dy*4 + dx
-        for (int n = 0; n < 32; ++n)
-            for (int e = 0; e < 8; ++e) {
-                uint16_t s2[2];
-                host_split2(c1w[n * 16 + 8 * c2 + e] * TC_SCALE_W, s2);
-                for (int s = 0; s < 2; ++s) p1[((size_t)c2 * 64 + s * 32 + n) * 8 + e] = s2[s];
-            }
-    for (int dy = 0; dy < 4; ++dy)                               // conv2: [(dy, half)][split][chunk][n = dx*32 + cout][8]
-        for (int hh = 0; hh < 2; ++hh)
-            for (int c2 = 0; c2 < 2; ++c2)
-                for (int dx = 0; dx < 4; ++dx)
-                    for (int n = 0; n < 32; ++n)
-                        for (int e = 0; e < 8; ++e) {
-                            const int ci = 16 * hh + 8 * c2 + e;
-                            uint16_t s2[2];
-                            host_split2(c2w[(n * 32 + ci) * 16 + dy * 4 + dx] * TC_SCALE_W, s2);
-                            for (int s = 0; s < 2; ++s) p2[(((((size_t)(dy * 2 + hh)) * 2 + s) * 2 + c2) * 128 + dx * 32 + n) * 8 + e] = s2[s];
-                        }
-    for (int j = 0; j < TDF_KBLOCKS; ++j)                        // fc1: k' = pixel*32 + channel, pixel = y*4 + x; torch k = c*64 + pixel
-        for (int c2 = 0; c2 < 2; ++c2)
-            for (int n = 0; n < 128; ++n)
-                for (int e = 0; e < 8; ++e) {
-                    const int kp = j * 16 + c2 * 8 + e, p = kp >> 5, c = kp & 31;
-                    uint16_t s2[2];
-                    host_split2(f1w[(size_t)n * 2048 + c * 64 + p] * TC_SCALE_W, s2);
-                    for (int s = 0; s < 2; ++s) pf[((((size_t)s * TDF_KBLOCKS + j) * 2 + c2) * 128 + n) * 8 + e] = s2[s];
-                }
-    if (!st->d_w && cudaMalloc(&st->d_w, h.size()) != cudaSuccess) return 1;
-    if (cudaMemcpyAsync(st->d_w, h.data(), h.size(), cudaMemcpyHostToDevice, stream) != cudaSuccess) return 1;
+    std::vector<uint8_t> h(DN_TC_PACKED_BYTES);
+    TW.wc1 = d_w; TW.wc2 = d_w + TDC_W1BYTES; TW.wfc = TW.wc2 + TDC_WBYTES;
+    auto at = [&](const uint8_t *d) { return reinterpret_cast<uint16_t *>(h.data() + (d - d_w)); };
+    pack_conv1(c1w, 16, at(TW.wc1));
+    pack_conv_shift(c2w, 4, at(TW.wc2));
+    pack_fc1(f1w, TdfPipe::N, TdfPipe::KBLOCKS, at(TW.wfc));
+    if (cudaMemcpyAsync(d_w, h.data(), h.size(), cudaMemcpyHostToDevice, stream) != cudaSuccess) return 1;
     if (cudaStreamSynchronize(stream) != cudaSuccess) return 1;
-    st->TW.wc1 = st->d_w; st->TW.wc2 = st->d_w + TDC_W1BYTES; st->TW.wfc = st->TW.wc2 + TDC_WBYTES;
     if (cudaFuncSetAttribute(k_tdc_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, TDC_SMEM) != cudaSuccess) return 1;
     if (cudaFuncSetAttribute(k_tdc_fc, cudaFuncAttributeMaxDynamicSharedMemorySize, TDF_SMEM) != cudaSuccess) return 1;
     return 0;
-}
-
-static int dn_tc_ensure_act2(DnTcState *st, size_t max_rows, cudaStream_t stream, bool *moved) {
-    size_t tiles = (max_rows + 127) / 128;
-    if (st->tiles >= tiles) return 0;
-    if (st->d_act2) { cudaStreamSynchronize(stream); cudaFree(st->d_act2); st->d_act2 = nullptr; if (moved) *moved = true; }
-    size_t bytes = (size_t)2 * tiles * DACT2_KCHUNKS * 2048;
-    if (cudaMalloc(&st->d_act2, bytes) != cudaSuccess) return 1;
-    cudaMemsetAsync(st->d_act2, 0, bytes, stream);
-    st->tiles = tiles;
-    return 0;
-}
-
-static void dn_tc_destroy(void *state) {
-    DnTcState *st = (DnTcState *)state;
-    if (!st) return;
-    cudaFree(st->d_w); cudaFree(st->d_act2);
-    delete st;
 }
 
 }  // namespace b200

@@ -15,10 +15,10 @@
 //              two lane shuffles.  tcgen05.mma (M=128 pixels, K=16) issued by one thread, accumulators in TMEM,
 //              completion through tcgen05.commit -> mbarrier; epilogues read TMEM with tcgen05.ld, apply bias+ReLU,
 //              re-split (fp16 x2) and write the next layer's operand (or act3 to HBM in the FC kernel's tile layout).
-//   k_tc_fc    [R,1792] x [1792,256]: 128-row tiles, operands streamed by cp.async.bulk (1-D TMA) into a 5-stage
-//              mbarrier ring — both operands are stored in HBM already in the canonical UMMA layout, so one bulk copy
-//              per operand block needs no tensor map; warp-specialised (producer / MMA issuer / 4 epilogue warps);
-//              epilogue fuses bias+ReLU+fc_out+sigmoid+affine and scatters (v, var) to the requesting tree slot.
+//   k_tc_fc    [R,1792] x [1792,256] on the FC pipeline it shares with k_tdc_fc (fc_pipeline below: 128-row tiles, operands
+//              streamed by cp.async.bulk (1-D TMA) into an 8-stage mbarrier ring — both operands are stored in HBM already in the
+//              canonical UMMA layout, so one bulk copy per operand block needs no tensor map; producer / MMA issuer / 4 epilogue
+//              warps); its epilogue fuses bias+ReLU+fc_out+sigmoid+affine and scatters (v, var) to the requesting tree slot.
 #pragma once
 #include <cuda_fp16.h>
 #include "search_dev.cuh"
@@ -203,10 +203,10 @@ static_assert(TCC_SMEM <= 227 * 1024, "k_tc_conv shared memory");
 struct TcWeights {
     const uint8_t *wc1;         // TCC_W1BYTES
     const uint8_t *wc2, *wc3;   // TCC_WBYTES each, already in the shared-memory layout
-    const uint8_t *wfc;         // [split 3][k16 block 112][chunk 2][n 256][16 B]
+    const uint8_t *wfc;         // [split 2][k16 block 112][chunk 2][n 256][16 B]
 };
 
-// act3 in HBM, FC-tile layout: [split][tile of 128 rows][k chunk 224][row 128][8 bf16], k' = (y*4 + x)*32 + c
+// act3 in HBM, FC-tile layout: [split][tile of 128 rows][k chunk 224][row 128][8 fp16], k' = (y*4 + x)*32 + c
 __device__ __forceinline__ size_t act3_off(int split, int n_tiles, int ridx, int kchunk) {
     return ((((size_t)split * n_tiles + (ridx >> 7)) * ACT3_KCHUNKS + kchunk) * 128 + (ridx & 127)) * 16;
 }
@@ -546,38 +546,46 @@ k_tc_conv(NetWeights W, TcWeights TW, const uint2 *req, const int32_t *n_req_ptr
     if (warp == TCC_ISSUER) tmem_dealloc<TCC_TMEM_COLS>(tmem_base);
 }
 
-// ---------------------------------------------------------------------------------------------------- fc kernel
-constexpr int TCF_THREADS = 192;            // warp 0 producer, warp 1 MMA issuer, warps 2-5 epilogue
-constexpr int TCF_STAGES = 8;
-constexpr int TCF_A_BYTES = 2 * 128 * 16;   // one split of one k16 block of the A tile
-constexpr int TCF_B_BYTES = 2 * 256 * 16;
-constexpr int TCF_STAGE = 2 * TCF_A_BYTES + 2 * TCF_B_BYTES;   // 24576
-constexpr int TCF_KBLOCKS = 112;            // 1792 / 16
-constexpr int TCF_OFF_BAR = TCF_STAGES * TCF_STAGE;
-constexpr int TCF_OFF_EPI = TCF_OFF_BAR + 256;                 // (2*stages + 2 mbarriers + tmem ptr fit in 256 B) bias[256] | wout[2][256] | bout/ub/lb
-static_assert((2 * TCF_STAGES + 2) * 8 + 4 <= 256, "barrier block overflows into the epilogue constants");
-constexpr int TCF_SMEM = TCF_OFF_EPI + (256 * 3 + 8) * 4;
-constexpr int TCF_TMEM_COLS = 256;
+// ---------------------------------------------------------------------------------------------------- fc pipeline
+// [R, 16*KBLOCKS] x [16*KBLOCKS, N] over 128-row tiles, shared by k_tc_fc and k_tdc_fc.  Both operands are stored in HBM already in the
+// canonical UMMA layout (A: the conv kernel's output, [split 2][tile][k chunk][row 128][8 fp16]; B: the packed fc1 weights), so one
+// cp.async.bulk (1-D TMA) per operand block needs no tensor map.  Warp 0 streams the blocks into a STAGES-deep mbarrier ring, one lane
+// of warp 1 issues three split MMAs per k block into N TMEM columns, warps 2-5 run the network's epilogue on the finished accumulator.
+constexpr int FC_PIPE_THREADS = 192;
+template <int N_, int KBLOCKS_, int STAGES_>
+struct FcPipe {
+    static constexpr int N = N_, KBLOCKS = KBLOCKS_, KCHUNKS = 2 * KBLOCKS, STAGES = STAGES_, TMEM_COLS = N;
+    static constexpr int A_BYTES = 2 * 128 * 16;                 // one split of one k16 block of the A tile
+    static constexpr int B_BYTES = 2 * N * 16;
+    static constexpr int STAGE = 2 * A_BYTES + 2 * B_BYTES;
+    static constexpr int OFF_BAR = STAGES * STAGE;
+    static constexpr int OFF_EPI = OFF_BAR + 256;                 // the epilogue's constants
+    static_assert((2 * STAGES + 2) * 8 + 4 <= 256, "barrier block overflows into the epilogue constants");
+    static constexpr size_t ACT_TILE_BYTES = (size_t)2 * KCHUNKS * 2048;   // one 128-row tile of the A operand, both splits
+};
 
-__global__ void __launch_bounds__(TCF_THREADS, 1)
-k_tc_fc(NetWeights W, TcWeights TW, const uint8_t *act3, int n_tiles_alloc, const uint2 *req, const int32_t *n_req_ptr, float2 *eval_out) {
+// load_consts(t) copies the epilogue's constants to shared memory (thread t of FC_PIPE_THREADS).  epi(taddr, tile, row, n_req, drained) runs
+// once per tile in every epilogue thread: taddr is the TMEM address of the thread's accumulator row, which holds request
+// tile * 128 + row (>= n_req in the last tile's padding); it calls drained() once it has read the accumulator.
+template <class P, class LoadConsts, class Epi>
+__device__ __forceinline__ void fc_pipeline(const uint8_t *act, int n_tiles_alloc, const uint8_t *wfc, const int32_t *n_req_ptr,
+                                            LoadConsts load_consts, Epi epi) {
     extern __shared__ __align__(128) uint8_t smem[];
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem + TCF_OFF_BAR);     // [stage] operands landed
-    uint64_t *empty = full + TCF_STAGES;                                    // [stage] operands consumed
-    uint64_t *acc_full = empty + TCF_STAGES;                                // accumulator complete
-    uint64_t *acc_empty = acc_full + 1;                                     // accumulator drained by the epilogue
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem + P::OFF_BAR);   // [stage] operands landed
+    uint64_t *empty = full + P::STAGES;                                  // [stage] operands consumed
+    uint64_t *acc_full = empty + P::STAGES;                              // accumulator complete
+    uint64_t *acc_empty = acc_full + 1;                                  // accumulator drained by the epilogue
     uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(acc_empty + 1);
-    float *sBias = reinterpret_cast<float *>(smem + TCF_OFF_EPI), *sWo = sBias + 256, *sTail = sWo + 512;
     const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-    for (int i = t; i < 256; i += TCF_THREADS) { sBias[i] = W.bfc1[i]; sWo[i] = W.wout[i]; sWo[256 + i] = W.wout[256 + i]; }
-    if (t < 2) { sTail[t] = W.bout[t]; sTail[2 + t] = W.ub[t]; sTail[4 + t] = W.lb[t]; }
+    __builtin_assume(t < FC_PIPE_THREADS);   // the kernels' launch bounds, which an inlined function does not see
+    load_consts(t);
     if (t == 0) {
-        for (int i = 0; i < TCF_STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+        for (int i = 0; i < P::STAGES; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
         mbar_init(acc_full, 1);
         mbar_init(acc_empty, 128);
         fence_barrier_init();
     }
-    if (warp == 1) tmem_alloc<TCF_TMEM_COLS>(tmem_ptr);
+    if (warp == 1) tmem_alloc<P::TMEM_COLS>(tmem_ptr);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -588,41 +596,41 @@ k_tc_fc(NetWeights W, TcWeights TW, const uint8_t *act3, int n_tiles_alloc, cons
         if (lane == 0) {   // ===== producer: bulk copies of the pre-laid-out operand blocks
             int stage = 0; uint32_t ph = 0;
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-                for (int j = 0; j < TCF_KBLOCKS; ++j) {
+                for (int j = 0; j < P::KBLOCKS; ++j) {
                     mbar_wait(&empty[stage], ph ^ 1);
-                    mbar_expect_tx(&full[stage], TCF_STAGE);
-                    uint8_t *dst = smem + stage * TCF_STAGE;
+                    mbar_expect_tx(&full[stage], P::STAGE);
+                    uint8_t *dst = smem + stage * P::STAGE;
 #pragma unroll
                     for (int s = 0; s < 2; ++s) {
-                        bulk_g2s(dst + s * TCF_A_BYTES, act3 + (((size_t)s * n_tiles_alloc + tile) * ACT3_KCHUNKS + 2 * j) * 2048, TCF_A_BYTES, &full[stage]);
-                        bulk_g2s(dst + 2 * TCF_A_BYTES + s * TCF_B_BYTES, TW.wfc + ((size_t)s * TCF_KBLOCKS + j) * TCF_B_BYTES, TCF_B_BYTES, &full[stage]);
+                        bulk_g2s(dst + s * P::A_BYTES, act + (((size_t)s * n_tiles_alloc + tile) * P::KCHUNKS + 2 * j) * 2048, P::A_BYTES, &full[stage]);
+                        bulk_g2s(dst + 2 * P::A_BYTES + s * P::B_BYTES, wfc + ((size_t)s * P::KBLOCKS + j) * P::B_BYTES, P::B_BYTES, &full[stage]);
                     }
-                    if (++stage == TCF_STAGES) { stage = 0; ph ^= 1; }
+                    if (++stage == P::STAGES) { stage = 0; ph ^= 1; }
                 }
             }
         }
     } else if (warp == 1) {
-        if (lane == 0) {   // ===== MMA issuer: D[128 x 256] += A[128 x 16] * B[256 x 16]^T, six split terms per k block
-            const uint32_t idesc = umma_idesc_f16(128, 256);
+        if (lane == 0) {   // ===== MMA issuer: D[128 x N] += A[128 x 16] * B[N x 16]^T, three split terms per k block
+            const uint32_t idesc = umma_idesc_f16(128, P::N);
             int stage = 0; uint32_t ph = 0, aph = 0;
             for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 mbar_wait(acc_empty, aph ^ 1);
                 tc_fence_after();
                 uint32_t acc = 0;
-                for (int j = 0; j < TCF_KBLOCKS; ++j) {
+                for (int j = 0; j < P::KBLOCKS; ++j) {
                     mbar_wait(&full[stage], ph);
                     tc_fence_after();
-                    const uint32_t sbase = smem_u32(smem + stage * TCF_STAGE);
+                    const uint32_t sbase = smem_u32(smem + stage * P::STAGE);
 #pragma unroll
                     for (int term = 0; term < 3; ++term) {   // a1*b2, a2*b1, a1*b1 (small terms first)
                         const int sa = term == 1 ? 1 : 0, sb = term == 0 ? 1 : 0;
-                        uint64_t ad = umma_desc(sbase + sa * TCF_A_BYTES, 128 * 16, 128);
-                        uint64_t bd = umma_desc(sbase + 2 * TCF_A_BYTES + sb * TCF_B_BYTES, 256 * 16, 128);
+                        uint64_t ad = umma_desc(sbase + sa * P::A_BYTES, 128 * 16, 128);
+                        uint64_t bd = umma_desc(sbase + 2 * P::A_BYTES + sb * P::B_BYTES, P::N * 16, 128);
                         umma_f16(tmem_base, ad, bd, idesc, acc);
                         acc = 1;
                     }
                     umma_commit(&empty[stage]);
-                    if (++stage == TCF_STAGES) { stage = 0; ph ^= 1; }
+                    if (++stage == P::STAGES) { stage = 0; ph ^= 1; }
                 }
                 umma_commit(acc_full);
                 aph ^= 1;
@@ -634,42 +642,53 @@ k_tc_fc(NetWeights W, TcWeights TW, const uint8_t *act3, int n_tiles_alloc, cons
         for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
             mbar_wait(acc_full, aph);
             tc_fence_after();
-            float p0 = 0.f, p1 = 0.f;
-#pragma unroll 1
-            for (int c0 = 0; c0 < 256; c0 += 16) {
-                float v[16];
-                tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + c0, v);
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    float h = fmaxf(v[j] * TC_UNSCALE + sBias[c0 + j], 0.f);   // model_vv.py:39-40
-                    p0 = fmaf(h, sWo[c0 + j], p0); p1 = fmaf(h, sWo[256 + c0 + j], p1);   // :41
-                }
-            }
-            tc_fence_before();
-            mbar_arrive(acc_empty);
-            const int ridx = tile * 128 + row;
-            if (ridx < n_req) {
-                float x0 = p0 + sTail[0], x1 = p1 + sTail[1];
-                float s0 = 1.f / (1.f + expf(-x0)), s1 = 1.f / (1.f + expf(-x1));      // :42
-                uint2 rq = req[ridx];
-                eval_out[(size_t)rq.x * 8 + (rq.y >> 28)] =
-                    make_float2(__fadd_rn(__fmul_rn(s0, sTail[2]), sTail[4]), __fadd_rn(__fmul_rn(s1, sTail[3]), sTail[5]));   // :51
-            }
+            epi(tmem_base + ((uint32_t)(q * 32) << 16), tile, row, n_req, [&] { tc_fence_before(); mbar_arrive(acc_empty); });
             aph ^= 1;
         }
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 1) tmem_dealloc<TCF_TMEM_COLS>(tmem_base);
+    if (warp == 1) tmem_dealloc<P::TMEM_COLS>(tmem_base);
 }
 
-// ---------------------------------------------------------------------------------------------------- host side
-struct TcState {
-    uint8_t *d_w = nullptr;      // wc1 | wc2 | wc3 | wfc
-    TcWeights TW{};
-    uint8_t *d_act3 = nullptr; size_t tiles = 0;
-};
+// ---------------------------------------------------------------------------------------------------- fc kernel
+using TcfPipe = FcPipe<256, ACT3_KCHUNKS / 2, 8>;
+constexpr int TCF_SMEM = TcfPipe::OFF_EPI + (256 * 3 + 8) * 4;          // bias[256] | wout[2][256] | bout/ub/lb
 
+__global__ void __launch_bounds__(FC_PIPE_THREADS, 1)
+k_tc_fc(NetWeights W, TcWeights TW, const uint8_t *act3, int n_tiles_alloc, const uint2 *req, const int32_t *n_req_ptr, float2 *eval_out) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    float *sBias = reinterpret_cast<float *>(smem + TcfPipe::OFF_EPI), *sWo = sBias + 256, *sTail = sWo + 512;
+    auto load_consts = [&](int t) {
+        for (int i = t; i < 256; i += FC_PIPE_THREADS) { sBias[i] = W.bfc1[i]; sWo[i] = W.wout[i]; sWo[256 + i] = W.wout[256 + i]; }
+        if (t < 2) { sTail[t] = W.bout[t]; sTail[2 + t] = W.ub[t]; sTail[4 + t] = W.lb[t]; }
+    };
+    fc_pipeline<TcfPipe>(act3, n_tiles_alloc, TW.wfc, n_req_ptr, load_consts, [&](uint32_t taddr, int tile, int row, int n_req, auto drained) {
+        float p0 = 0.f, p1 = 0.f;
+#pragma unroll 1
+        for (int c0 = 0; c0 < 256; c0 += 16) {
+            float v[16];
+            tmem_ld16(taddr + c0, v);
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                float h = fmaxf(v[j] * TC_UNSCALE + sBias[c0 + j], 0.f);   // model_vv.py:39-40
+                p0 = fmaf(h, sWo[c0 + j], p0); p1 = fmaf(h, sWo[256 + c0 + j], p1);   // :41
+            }
+        }
+        drained();
+        const int ridx = tile * 128 + row;
+        if (ridx < n_req) {
+            float x0 = p0 + sTail[0], x1 = p1 + sTail[1];
+            float s0 = 1.f / (1.f + expf(-x0)), s1 = 1.f / (1.f + expf(-x1));      // :42
+            uint2 rq = req[ridx];
+            eval_out[(size_t)rq.x * 8 + (rq.y >> 28)] =
+                make_float2(__fadd_rn(__fmul_rn(s0, sTail[2]), sTail[4]), __fadd_rn(__fmul_rn(s1, sTail[3]), sTail[5]));   // :51
+        }
+    });
+}
+
+// ---------------------------------------------------------------------------------------------------- host side: weight packing
+// Pure re-layout + fp16 splitting of the state_dict-order weights, shared by both tensor-core networks.
 static inline void host_split2(float x, uint16_t *o) {   // x*scale = h1 + h2 in fp16
     __half h1 = __float2half_rn(x);
     __half h2 = __float2half_rn(x - __half2float(h1));
@@ -677,74 +696,67 @@ static inline void host_split2(float x, uint16_t *o) {   // x*scale = h1 + h2 in
 }
 static inline float host_half_f(uint16_t h) { __half x; memcpy(&x, &h, 2); return __half2float(x); }
 
-// w = the state_dict-order weight vector of include/b200_tetris_mcts.h.  Pure re-layout + bf16 splitting.
-static int tc_prepare(void **state, const float *w, cudaStream_t stream) {
-    TcState *st = (TcState *)*state;
-    if (!st) { st = new TcState(); *state = st; }
-    const float *c1w = w, *c2w = w + 288 + 32, *c3w = c2w + 9216 + 32, *f1w = c3w + 9216 + 32;
-    const size_t fc_bytes = (size_t)2 * TCF_KBLOCKS * TCF_B_BYTES;
-    std::vector<uint8_t> h(TCC_W1BYTES + 2 * (size_t)TCC_WBYTES + fc_bytes);
-    uint16_t *p1 = reinterpret_cast<uint16_t *>(h.data());
-    uint16_t *p2 = reinterpret_cast<uint16_t *>(h.data() + TCC_W1BYTES), *p3 = reinterpret_cast<uint16_t *>(h.data() + TCC_W1BYTES + TCC_WBYTES);
-    uint16_t *pf = reinterpret_cast<uint16_t *>(h.data() + TCC_W1BYTES + 2 * (size_t)TCC_WBYTES);
-    for (int c2 = 0; c2 < 2; ++c2)                               // conv1: [chunk][n = split*32 + cout][8], k = tap
+// conv1 (1 -> 32) as one K = 16 im2col MMA: [chunk 2][n = split*32 + cout][8], k = tap (9 or 16 taps; the rest zero)
+static void pack_conv1(const float *cw, int taps, uint16_t *dst) {
+    for (int c2 = 0; c2 < 2; ++c2)
         for (int n = 0; n < 32; ++n)
             for (int e = 0; e < 8; ++e) {
                 const int tap = 8 * c2 + e;
                 uint16_t s2[2] = {0, 0};
-                if (tap < 9) host_split2(c1w[n * 9 + tap] * TC_SCALE_W, s2);
-                for (int s = 0; s < 2; ++s) p1[((size_t)c2 * 64 + s * 32 + n) * 8 + e] = s2[s];
+                if (tap < taps) host_split2(cw[n * taps + tap] * TC_SCALE_W, s2);
+                for (int s = 0; s < 2; ++s) dst[((size_t)c2 * 64 + s * 32 + n) * 8 + e] = s2[s];
             }
-    for (int layer = 0; layer < 2; ++layer) {                    // conv2/3: [(dy, half)][split][chunk][n = dx*32 + cout][8]
-        const float *cw = layer ? c3w : c2w;
-        uint16_t *dst = layer ? p3 : p2;
-        for (int dy = 0; dy < 3; ++dy)
-            for (int hh = 0; hh < 2; ++hh)
-                for (int c2 = 0; c2 < 2; ++c2)
-                    for (int dx = 0; dx < 3; ++dx)
-                        for (int n = 0; n < 32; ++n)
-                            for (int e = 0; e < 8; ++e) {
-                                int ci = 16 * hh + 8 * c2 + e;
-                                uint16_t s2[2];
-                                host_split2(cw[(n * 32 + ci) * 9 + dy * 3 + dx] * TC_SCALE_W, s2);
-                                for (int s = 0; s < 2; ++s)   // dy shifts the A operand and selects the block, dx is stacked along N
-                                    dst[(((((size_t)(dy * 2 + hh)) * 2 + s) * 2 + c2) * 96 + dx * 32 + n) * 8 + e] = s2[s];
-                            }
-    }
-    for (int j = 0; j < TCF_KBLOCKS; ++j)
+}
+
+// a taps x taps conv (32 -> 32) as a shift-GEMM: [(dy, half)][split][chunk][n = dx*32 + cout][8], N = taps * 32 (96 or 128)
+static void pack_conv_shift(const float *cw, int taps, uint16_t *dst) {
+    const int N = taps * 32;
+    for (int dy = 0; dy < taps; ++dy)
+        for (int hh = 0; hh < 2; ++hh)
+            for (int c2 = 0; c2 < 2; ++c2)
+                for (int dx = 0; dx < taps; ++dx)
+                    for (int n = 0; n < 32; ++n)
+                        for (int e = 0; e < 8; ++e) {
+                            const int ci = 16 * hh + 8 * c2 + e;
+                            uint16_t s2[2];
+                            host_split2(cw[(n * 32 + ci) * taps * taps + dy * taps + dx] * TC_SCALE_W, s2);
+                            for (int s = 0; s < 2; ++s)   // dy shifts the A operand and selects the block, dx is stacked along N
+                                dst[(((((size_t)(dy * 2 + hh)) * 2 + s) * 2 + c2) * N + dx * 32 + n) * 8 + e] = s2[s];
+                        }
+}
+
+// fc1 [N][K] with torch's flatten order k = c*pixels + p (32 channels, pixels = K / 32) as fc_pipeline's B operand:
+// [split][k16 block][chunk][n][8], k' = pixel*32 + channel
+static void pack_fc1(const float *fw, int N, int kblocks, uint16_t *dst) {
+    const int K = kblocks * 16, pixels = K / 32;
+    for (int j = 0; j < kblocks; ++j)
         for (int c2 = 0; c2 < 2; ++c2)
-            for (int n = 0; n < 256; ++n)
+            for (int n = 0; n < N; ++n)
                 for (int e = 0; e < 8; ++e) {
-                    int kp = j * 16 + c2 * 8 + e, p = kp >> 5, c = kp & 31;      // k' = pixel*32 + channel, pixel = y*4 + x
+                    const int kp = j * 16 + c2 * 8 + e, p = kp >> 5, c = kp & 31;
                     uint16_t s2[2];
-                    host_split2(f1w[(size_t)n * 1792 + c * 56 + p] * TC_SCALE_W, s2);
-                    for (int s = 0; s < 2; ++s) pf[((((size_t)s * TCF_KBLOCKS + j) * 2 + c2) * 256 + n) * 8 + e] = s2[s];
+                    host_split2(fw[(size_t)n * K + c * pixels + p] * TC_SCALE_W, s2);
+                    for (int s = 0; s < 2; ++s) dst[((((size_t)s * kblocks + j) * 2 + c2) * N + n) * 8 + e] = s2[s];
                 }
-    if (!st->d_w && cudaMalloc(&st->d_w, h.size()) != cudaSuccess) return 1;
-    if (cudaMemcpyAsync(st->d_w, h.data(), h.size(), cudaMemcpyHostToDevice, stream) != cudaSuccess) return 1;
+}
+
+constexpr size_t TC_PACKED_BYTES = TCC_W1BYTES + 2 * (size_t)TCC_WBYTES + (size_t)2 * TcfPipe::KBLOCKS * TcfPipe::B_BYTES;   // wc1 | wc2 | wc3 | wfc
+
+// w = the state_dict-order weight vector of include/b200_tetris_mcts.h, packed into d_w (TC_PACKED_BYTES)
+static int tc_prepare(const float *w, uint8_t *d_w, TcWeights &TW, cudaStream_t stream) {
+    const float *c1w = w, *c2w = w + 288 + 32, *c3w = c2w + 9216 + 32, *f1w = c3w + 9216 + 32;
+    std::vector<uint8_t> h(TC_PACKED_BYTES);
+    TW.wc1 = d_w; TW.wc2 = d_w + TCC_W1BYTES; TW.wc3 = TW.wc2 + TCC_WBYTES; TW.wfc = TW.wc3 + TCC_WBYTES;
+    auto at = [&](const uint8_t *d) { return reinterpret_cast<uint16_t *>(h.data() + (d - d_w)); };
+    pack_conv1(c1w, 9, at(TW.wc1));
+    pack_conv_shift(c2w, 3, at(TW.wc2));
+    pack_conv_shift(c3w, 3, at(TW.wc3));
+    pack_fc1(f1w, TcfPipe::N, TcfPipe::KBLOCKS, at(TW.wfc));
+    if (cudaMemcpyAsync(d_w, h.data(), h.size(), cudaMemcpyHostToDevice, stream) != cudaSuccess) return 1;
     if (cudaStreamSynchronize(stream) != cudaSuccess) return 1;
-    st->TW.wc1 = st->d_w; st->TW.wc2 = st->d_w + TCC_W1BYTES; st->TW.wc3 = st->TW.wc2 + TCC_WBYTES; st->TW.wfc = st->TW.wc3 + TCC_WBYTES;
     if (cudaFuncSetAttribute(k_tc_conv, cudaFuncAttributeMaxDynamicSharedMemorySize, TCC_SMEM) != cudaSuccess) return 1;
     if (cudaFuncSetAttribute(k_tc_fc, cudaFuncAttributeMaxDynamicSharedMemorySize, TCF_SMEM) != cudaSuccess) return 1;
     return 0;
-}
-
-static int tc_ensure_act3(TcState *st, size_t max_rows, cudaStream_t stream) {
-    size_t tiles = (max_rows + 127) / 128;
-    if (st->tiles >= tiles) return 0;
-    if (st->d_act3) { cudaStreamSynchronize(stream); cudaFree(st->d_act3); st->d_act3 = nullptr; }
-    size_t bytes = (size_t)2 * tiles * ACT3_KCHUNKS * 2048;
-    if (cudaMalloc(&st->d_act3, bytes) != cudaSuccess) return 1;
-    cudaMemsetAsync(st->d_act3, 0, bytes, stream);
-    st->tiles = tiles;
-    return 0;
-}
-
-static void tc_destroy(void *state) {
-    TcState *st = (TcState *)state;
-    if (!st) return;
-    cudaFree(st->d_w); cudaFree(st->d_act3);
-    delete st;
 }
 
 }  // namespace b200
